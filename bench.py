@@ -4,6 +4,7 @@
 bench.py — gp.compute() + gp.log_likelihood() throughput (N-points/s) for the HODLR path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg3|cfg2|cfg5]
+                    [--dump-outputs DIR]
 
 One "step" = one gp.compute(x, yerr) + one gp.log_likelihood(y) on a fixed synthetic data set (SURVEY.md §8d):
     x = sort(U(0, 10*N/1000)) (rng 1234), yerr = 0.1, y = sin(x) + 0.1*N(0,1).
@@ -21,6 +22,11 @@ mt19937, dense storage of exhausted blocks) at a small N.
 
 JSON keys follow the driver contract; extra: roofline{}, cpu_baseline{}, clocks{}, e2e{}, gpu_launches, same_n{},
 kernel_ms{}, secondary{cfg2, cfg4}.
+
+`--dump-outputs DIR` writes what the last timed step returned, as float64 arrays of shape (1,): log_likelihood.npy,
+log_determinant.npy and dot_solve.npy (y^T K^-1 y) of the device-resident leg, and log_likelihood_e2e.npy of the
+public-API leg.  The inputs are seeded, so two builds run with the same arguments can be compared output for output.
+Two runs of one build agreed to 4e-16 relative, not bit for bit (B200, 1000 W power limit), so compare with a tolerance.
 """
 import argparse
 import ctypes as C
@@ -36,6 +42,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only: nothing is written next to the sources
 
 # FP64 peaks of this pool's B200, BUILDER-measured with tools/fp64_peaks.cu (profiles/fp64_peaks_r01.txt); the
 # driver-written MEASURED_PEAKS.json has only HBM and bf16 entries.  cuBLAS dgemm reaches 35.4 TFLOP/s on the same box.
@@ -232,6 +239,7 @@ class DeviceLeg(object):
         ld, out = C.c_double(), C.c_double()
         _lib.check(lib.bgp_hodlr_log_determinant(self.native._ptr, C.byref(ld)))
         _lib.check(lib.bgp_hodlr_dot_solve_dev(self.native._ptr, dy, C.byref(out)))
+        self.last = {"log_determinant": ld.value, "dot_solve": out.value}
         return -0.5 * (n * np.log(2 * np.pi) + ld.value) - 0.5 * out.value
 
     def close(self):
@@ -330,6 +338,12 @@ def dense_secondary(lib, flush_l2, barrier, reps=2):
     return out
 
 
+def dump_outputs(directory, outputs):
+    os.makedirs(directory, exist_ok=True)
+    for name, v in outputs.items():
+        np.save(os.path.join(directory, name + ".npy"), np.array([v], dtype=np.float64))
+
+
 def run_ours(args):
     import torch
     from george_b200 import _lib, GP, HODLRSolver
@@ -377,9 +391,12 @@ def run_ours(args):
         from george_b200.parallel import ShardedHODLRSolver
         sharded = ShardedHODLRSolver(kernel, **solver_kw)
 
+        last = {}
+
         def step_value():
             sharded.compute(x[:, None], yerr)
-            return -0.5 * (n * np.log(2 * np.pi) + sharded.log_determinant) - 0.5 * sharded.dot_solve(y)
+            last.update(log_determinant=sharded.log_determinant, dot_solve=sharded.dot_solve(y))
+            return -0.5 * (n * np.log(2 * np.pi) + last["log_determinant"]) - 0.5 * last["dot_solve"]
         collect = None
 
     sampler = ClockSampler(local_rank)
@@ -391,6 +408,7 @@ def run_ours(args):
     launches0 = lib.bgp_launch_count()
     ll_value, t_steps, t_wall = time_steps(step_value, args.steps, 0, flush_l2, barrier, collect)
     launches = lib.bgp_launch_count() - launches0
+    outputs = dict(leg.last if world == 1 else last, log_likelihood=ll_value)
     total = sum(t_steps)
     if dist is not None:
         t = torch.tensor([total], dtype=torch.float64, device="cuda")
@@ -432,6 +450,9 @@ def run_ours(args):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         total_e2e = float(t.item())
     clocks = sampler.stop() if rank == 0 else None
+    outputs["log_likelihood_e2e"] = ll_e2e
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
 
     if rank != 0:
         if dist is not None:
@@ -600,7 +621,13 @@ def main():
     ap.add_argument("--exhaust", default="lowrank", choices=["dense", "lowrank"])
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-secondary", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step of the CUDA path to DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,34 +1,35 @@
 # -*- coding: utf-8 -*-
 """Every kernel instance of the reference's own suite (tests/test_kernels.py `kernels_to_test` + `test_stationary`):
-(CPU) our oracle == the reference's compiled kernel_interface, bit for bit, values and hyper-gradients;
+(CPU) our oracle == the reference's compiled kernel_interface, bit for bit, values and hyper-gradients (what it returned
+      is kept in tests/golden/reference_kernel_interface.npz);
 (GPU) the CUDA build == the oracle, and the reference's finite-difference gradient check passes on the device path."""
 import numpy as np
 import pytest
 
 from conftest import reference_kernel_list
+from test_oracle_kernels import assert_equals_reference_binary
 
 KERNELS = reference_kernel_list()
 IDS = ["{0:02d}-{1}".format(i, type(k).__name__) for i, k in enumerate(KERNELS)]
 
 
-@pytest.mark.parametrize("kernel", KERNELS, ids=IDS)
-def test_oracle_equals_reference_binary(oracle, kernel):
-    from george_b200._spec import flatten
-    ref = oracle.reference_kernel_interface()
-    if ref is None:
-        pytest.skip("oracle/_ref/kernel_interface*.so not built (needs /root/reference)")
+def kernel_list_input(kernel):
     np.random.seed(123)
-    t1 = np.random.randn(20, kernel.ndim)
+    return np.random.randn(20, kernel.ndim)
+
+
+@pytest.mark.parametrize("kid,kernel", list(zip(IDS, KERNELS)), ids=IDS)
+def test_oracle_equals_reference_binary(oracle, kid, kernel):
+    from george_b200._spec import flatten
+    t1 = kernel_list_input(kernel)
     spec = flatten(kernel)
-    r = ref.KernelInterface(kernel)
-    assert np.array_equal(oracle.value_symmetric(spec, t1), r.value_symmetric(t1))
-    assert np.array_equal(oracle.value_general(spec, t1, t1[:1]), r.value_general(t1, t1[:1]))
+    outs = [oracle.value_symmetric(spec, t1), oracle.value_general(spec, t1, t1[:1])]
     if kernel.full_size:
         which = np.ones(kernel.full_size, dtype=np.uint32)
-        assert np.array_equal(oracle.gradient_general(spec, which, t1, t1[:3]), r.gradient_general(which, t1, t1[:3]))
+        outs.append(oracle.gradient_general(spec, which, t1, t1[:3]))
     # input-coordinate gradients (kernel_interface.cpp:127-157)
-    assert np.array_equal(oracle.x_gradient_general(spec, 1, t1, t1[:3]), r.x1_gradient_general(t1, t1[:3]))
-    assert np.array_equal(oracle.x_gradient_general(spec, 2, t1[:3], t1), r.x2_gradient_general(t1[:3], t1))
+    outs += [oracle.x_gradient_general(spec, 1, t1, t1[:3]), oracle.x_gradient_general(spec, 2, t1[:3], t1)]
+    assert_equals_reference_binary("list", kid, outs)
 
 
 def test_stationary_constructor_errors():
