@@ -86,6 +86,36 @@ struct DevBuf {
   DevBuf& operator=(const DevBuf&) = delete;
 };
 
+// Owned stream / event, created on first use.  The destructor synchronises, then destroys.  A DevBuf is freed on its
+// stream, so an owner declares its Streams before its DevBufs (members are destroyed in reverse order).
+struct Stream {
+  cudaStream_t s = nullptr;
+  int create() {
+    if (!s) BGP_CUDA(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
+    return BGP_OK;
+  }
+  void sync() const { if (s) cudaStreamSynchronize(s); }
+  operator cudaStream_t() const { return s; }
+  ~Stream() { if (s) { cudaStreamSynchronize(s); cudaStreamDestroy(s); } }
+  Stream() {}
+  Stream(const Stream&) = delete;
+  Stream& operator=(const Stream&) = delete;
+};
+
+struct Event {
+  cudaEvent_t e = nullptr;
+  int create() {
+    if (!e) BGP_CUDA(cudaEventCreate(&e));
+    return BGP_OK;
+  }
+  operator cudaEvent_t() const { return e; }
+  ~Event() { if (e) { cudaEventSynchronize(e); cudaEventDestroy(e); } }
+  Event() {}
+  Event(Event&& o) noexcept : e(o.e) { o.e = nullptr; }  // (kept in a growing std::vector)
+  Event(const Event&) = delete;
+  Event& operator=(const Event&) = delete;
+};
+
 // ---------------------------------------------------------------------------------------------------------------
 // device side
 // ---------------------------------------------------------------------------------------------------------------

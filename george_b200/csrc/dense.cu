@@ -383,8 +383,9 @@ __global__ void apply_sqrt_kernel(const double* __restrict__ L, int64_t n, const
 using namespace bgp;
 
 struct bgp_dense {
-  cudaStream_t s = nullptr;
-  cudaEvent_t ev[4] = {nullptr};
+  Stream s;  // declared before every DevBuf: streams outlive buffers
+  Event ev[4];
+  ~bgp_dense() { s.sync(); }
   int64_t n = 0;
   bool computed = false;
   double log_det = 0.0;
@@ -400,35 +401,18 @@ struct bgp_dense {
   double t_ms[2] = {0, 0};
 };
 
-// outer block width (a multiple of DN_NB); BGP_DENSE_OB overrides the default for tuning runs
-static int64_t dense_outer_block() {
-  static int64_t ob = 0;
-  if (ob == 0) {
-    ob = DN_OB;
-    if (const char* e = getenv("BGP_DENSE_OB")) {
-      const long v = atol(e);
-      if (v >= DN_NB && v <= 4096 && v % DN_NB == 0) ob = v;
-    }
-  }
-  return ob;
+static int ensure_stream(bgp_dense* h) {
+  BGP_TRY(h->s.create());
+  for (Event& e : h->ev) BGP_TRY(e.create());
+  return BGP_OK;
 }
 
-// Blocked right-looking Cholesky with DELAYED trailing updates on three nested block sizes (64 | DN_MB | OB): after the
-// panel ending at column e, the rank-64 update touches only the rest of the current DN_MB block; when e closes a DN_MB
-// block its accumulated rank-DN_MB update touches the rest of the current OB block; when e closes an OB block the
-// rank-OB update touches everything to the right.  Almost all flops therefore run as GEMMs with K = OB, whose
+// Blocked right-looking Cholesky with DELAYED trailing updates on three nested block sizes (64 | DN_MB | DN_OB): after
+// the panel ending at column e, the rank-64 update touches only the rest of the current DN_MB block; when e closes a
+// DN_MB block its accumulated rank-DN_MB update touches the rest of the current DN_OB block; when e closes a DN_OB block
+// the rank-DN_OB update touches everything to the right.  Almost all flops therefore run as GEMMs with K = DN_OB, whose
 // read-modify-write epilogue of C is amortised over 16x more tensor work than at K = 64.
-static int64_t dense_mid_block(int64_t OB) {
-  static int64_t mb = 0;
-  if (mb == 0) {
-    mb = DN_MB;
-    if (const char* e = getenv("BGP_DENSE_MB")) {
-      const long v = atol(e);
-      if (v >= DN_NB && v % DN_NB == 0) mb = v;
-    }
-  }
-  return (mb < OB && OB % mb == 0) ? mb : OB;
-}
+static_assert(DN_MB % DN_NB == 0 && DN_MB < DN_OB && DN_OB % DN_MB == 0, "the three block sizes nest");
 
 static int dense_potrf(bgp_dense* h) {
   const int64_t n = h->n;
@@ -438,8 +422,6 @@ static int dense_potrf(bgp_dense* h) {
   std::vector<GemmDesc> descs;
   struct Step { int64_t k0; int nb; int64_t rem; int desc[3]; };
   std::vector<Step> steps;
-  const int64_t OB = dense_outer_block();
-  const int64_t MB = dense_mid_block(OB);
   // C[e:n, e:cend) -= L[e:n, b:e) L[e:cend, b:e)^T   (lower part only)
   auto add_update = [&](int64_t b, int64_t e, int64_t cend) -> int {
     if (e >= n || cend <= e || e <= b) return -1;
@@ -455,10 +437,10 @@ static int dense_potrf(bgp_dense* h) {
     Step st;
     st.k0 = j0; st.nb = (int)std::min<int64_t>(DN_NB, n - j0); st.rem = n - j0 - st.nb;
     const int64_t e = j0 + st.nb;
-    const int64_t mb0 = (j0 / MB) * MB, mb1 = std::min(n, mb0 + MB);  // the DN_MB block holding this panel
-    const int64_t ob0 = (j0 / OB) * OB, ob1 = std::min(n, ob0 + OB);  // the OB block holding it
+    const int64_t mb0 = (j0 / DN_MB) * DN_MB, mb1 = std::min<int64_t>(n, mb0 + DN_MB);  // the DN_MB block holding this panel
+    const int64_t ob0 = (j0 / DN_OB) * DN_OB, ob1 = std::min<int64_t>(n, ob0 + DN_OB);  // the DN_OB block holding it
     st.desc[0] = add_update(j0, e, mb1);
-    st.desc[1] = (e == mb1 && MB < OB) ? add_update(mb0, e, ob1) : -1;
+    st.desc[1] = (e == mb1) ? add_update(mb0, e, ob1) : -1;
     st.desc[2] = (e == ob1) ? add_update(ob0, e, n) : -1;
     steps.push_back(st);
   }
@@ -552,15 +534,6 @@ int bgp_dense_create(bgp_dense_t** out) {
 
 void bgp_dense_destroy(bgp_dense_t* h) {
   if (!h) return;
-  if (h->s) cudaStreamSynchronize(h->s);
-  h->d_prog.release(); h->d_x.release(); h->d_yerr.release(); h->d_diag.release(); h->d_A.release();
-  h->d_rhs.release(); h->d_scalar.release(); h->d_info.release(); h->d_gdesc.release();
-  h->d_tmp.release(); h->d_inv.release(); h->d_gscratch.release(); h->d_which.release();
-  if (h->s) {
-    cudaStreamSynchronize(h->s);
-    for (int i = 0; i < 4; ++i) cudaEventDestroy(h->ev[i]);
-    cudaStreamDestroy(h->s);
-  }
   delete h;
 }
 
@@ -569,10 +542,7 @@ int bgp_dense_compute(bgp_dense_t* h, const bgp_kernel_spec_t* spec, const doubl
   if (!h) { set_error("null handle"); return BGP_ERR_INVALID; }
   h->computed = false;
   BGP_TRY(require_device());
-  if (!h->s) {
-    BGP_CUDA(cudaStreamCreateWithFlags(&h->s, cudaStreamNonBlocking));
-    for (int i = 0; i < 4; ++i) BGP_CUDA(cudaEventCreate(&h->ev[i]));
-  }
+  BGP_TRY(ensure_stream(h));
   DevProgram P;
   BGP_TRY(build_dev_program(spec, &P));
   if (P.ndim != ndim) { set_error("dimension mismatch: kernel ndim %d, input ndim %d", P.ndim, ndim); return BGP_ERR_DIM; }
@@ -734,10 +704,7 @@ int bgp_dense_import_factor(bgp_dense_t* h, const double* factor, int64_t n, dou
   if (!h || n <= 0) { set_error("invalid argument"); return BGP_ERR_INVALID; }
   h->computed = false;
   BGP_TRY(require_device());
-  if (!h->s) {
-    BGP_CUDA(cudaStreamCreateWithFlags(&h->s, cudaStreamNonBlocking));
-    for (int i = 0; i < 4; ++i) BGP_CUDA(cudaEventCreate(&h->ev[i]));
-  }
+  BGP_TRY(ensure_stream(h));
   h->n = n;
   h->has_inputs = false;
   BGP_TRY(h->d_A.reserve((size_t)n * n, h->s));

@@ -36,7 +36,6 @@ using namespace bgp;
 
 struct HNode {
   int start, size, half, is_leaf, parent, dir, depth;
-  int slot;        // index within its level (internal) or within the leaf list
   int rank = 0, draws = 0, fallback = 0;
   int owned = 1;   // sharding: this process factors the node locally
   int top = 0;     // sharding: node above the shard cut (finished after the exchange)
@@ -66,9 +65,29 @@ struct AcaGraphKey {  // everything the captured ACA loop depends on
   int nn, ncc, nrc, shape, grid;
 };
 
+// the cached executable graph of the ACA loop (run_aca2) and the key it was captured for
+struct AcaGraph {
+  AcaGraphKey key;
+  cudaGraph_t graph = nullptr;
+  cudaGraphExec_t exec = nullptr;
+  void reset() {
+    if (exec) cudaGraphExecDestroy(exec);
+    if (graph) cudaGraphDestroy(graph);
+    exec = nullptr; graph = nullptr;
+  }
+  ~AcaGraph() { reset(); }
+  AcaGraph() {}
+  AcaGraph(const AcaGraph&) = delete;
+  AcaGraph& operator=(const AcaGraph&) = delete;
+};
+
 struct bgp_hodlr {
-  cudaStream_t sA = nullptr, sB = nullptr;
-  cudaEvent_t ev[8] = {nullptr};
+  // declared before every DevBuf: streams outlive buffers
+  Stream sA, sB, sC;  // sC: capture stream of the ACA graph
+  Event ev[8];
+  std::vector<Event> prof_events;
+  AcaGraph aca;
+  ~bgp_hodlr() { sA.sync(); sB.sync(); sC.sync(); }  // no buffer is freed while another stream still uses it
   int64_t n = 0;
   int ndim = 0;
   bgp_hodlr_opts_t opts;
@@ -80,8 +99,7 @@ struct bgp_hodlr {
   std::vector<int> leaves;   // pre-order ids
   std::vector<LevelInfo> levels;
   std::vector<int> piv_off;  // per internal node (by pre-order id) offset into pivot arrays, -1 for leaves
-  std::vector<int> h_piv_rows, h_piv_cols;
-  int max_leaf = 0, rtot = 0, vcols = 0, cut_depth = 0;
+  int max_leaf = 0, cut_depth = 0;
   int64_t row0 = 0, nloc = 0;
   std::vector<int64_t> shard_row0, shard_rows;
 
@@ -114,12 +132,7 @@ struct bgp_hodlr {
   DevBuf<unsigned long long> d_cmax, d_stats;
   DevBuf<int4> d_work;
   DevBuf<int> d_work_count, d_iter;
-  AcaGraphKey aca_key;
-  cudaGraph_t aca_graph = nullptr;
-  cudaGraphExec_t aca_exec = nullptr;
-  cudaStream_t sC = nullptr;  // capture stream
   bool profile = false;
-  std::vector<cudaEvent_t> prof_events;
   double prof[12] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};  // see bgp_hodlr_last_aca_profile
   DevBuf<double> d_vpart, d_upart, d_vmax;
   int aca_iters = 0;
@@ -130,11 +143,9 @@ struct bgp_hodlr {
 };
 
 static int ensure_streams(bgp_hodlr* h) {
-  if (!h->sA) {
-    BGP_CUDA(cudaStreamCreateWithFlags(&h->sA, cudaStreamNonBlocking));
-    BGP_CUDA(cudaStreamCreateWithFlags(&h->sB, cudaStreamNonBlocking));
-    for (int i = 0; i < 8; ++i) BGP_CUDA(cudaEventCreate(&h->ev[i]));
-  }
+  BGP_TRY(h->sA.create());
+  BGP_TRY(h->sB.create());
+  for (Event& e : h->ev) BGP_TRY(e.create());
   return BGP_OK;
 }
 
@@ -143,7 +154,6 @@ static void build_tree(bgp_hodlr* h, int start, int size, int dir, int parent, i
   HNode nd;
   nd.start = start; nd.size = size; nd.half = size / 2; nd.dir = dir; nd.parent = parent; nd.depth = depth;
   nd.is_leaf = !(nd.half >= h->opts.min_size);
-  nd.slot = 0;
   const int id = (int)h->nodes.size();
   h->nodes.push_back(nd);
   if (!nd.is_leaf) {
@@ -160,23 +170,12 @@ static int launch_leaf_solve(bgp_hodlr* h, double* X, int64_t ldx, const int* nc
                              int max_cols, cudaStream_t s) {
   const int nl = (int)h->leaves.size();
   if (nl == 0 || max_cols == 0) return BGP_OK;
-  // only leaves handled locally are in d_leaves.  Column groups of 8 by default.  BGP_LEAF_COLS=32 selects the 32-column
-  // instantiation for calls with more than 8 columns (the up-sweep): it streams the leaf factor once per 32 columns
-  // instead of once per 8, but measured SLOWER on the headline (up-sweep 3.39 vs 3.06 ms: four times the serial work per
-  // CTA at 128 registers, and the 512 MB of leaf factors mostly hit in the 126 MB L2 anyway) — kept as an experiment.
-  int wide = 0;
-  if (const char* e = getenv("BGP_LEAF_COLS")) wide = (atoi(e) > LS_COLS && max_cols > LS_COLS) ? 1 : 0;
-  const int cols = wide ? LS_COLS_WIDE : LS_COLS;
-  dim3 grid(nl, (max_cols + cols - 1) / cols);
-  const size_t smem = sizeof(double) * (size_t)h->max_leaf * cols;
+  // only leaves handled locally are in d_leaves; column groups of LS_COLS
+  dim3 grid(nl, (max_cols + LS_COLS - 1) / LS_COLS);
+  const size_t smem = sizeof(double) * (size_t)h->max_leaf * LS_COLS;
   if (smem > 200 * 1024) { set_error("leaf size %d too large for the leaf solve kernel", h->max_leaf); return BGP_ERR_INVALID; }
-  if (wide) {
-    cudaFuncSetAttribute(leaf_solve_kernel<LS_COLS_WIDE>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    leaf_solve_kernel<LS_COLS_WIDE><<<grid, LS_THREADS, smem, s>>>(h->d_leaves.p, h->d_L.p, X, ldx, ncols_by_depth, ncols_fixed, h->max_leaf);
-  } else {
-    cudaFuncSetAttribute(leaf_solve_kernel<LS_COLS>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    leaf_solve_kernel<LS_COLS><<<grid, LS_THREADS, smem, s>>>(h->d_leaves.p, h->d_L.p, X, ldx, ncols_by_depth, ncols_fixed, h->max_leaf);
-  }
+  cudaFuncSetAttribute(leaf_solve_kernel<LS_COLS>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+  leaf_solve_kernel<LS_COLS><<<grid, LS_THREADS, smem, s>>>(h->d_leaves.p, h->d_L.p, X, ldx, ncols_by_depth, ncols_fixed, h->max_leaf);
   BGP_LAUNCH_CHECK();
   return BGP_OK;
 }
@@ -291,11 +290,7 @@ static int run_aca2(bgp_hodlr* h, const std::vector<AcaDesc>& descs, std::vector
   if (nn == 0) return BGP_OK;
   std::vector<A2Node> hn(nn);
   std::vector<int> cchunk_node, rchunk_node;
-  int64_t cand_total = 0, top_cand_total = 0;
-  (void)top_cand_total;
-  // (the candidate scans of the nodes above the shard cut are done redundantly by every rank: with bound culling and
-  //  one-candidate batches they are cheap, and a collective inside the lock-step loop would put a latency on every step)
-  const bool dist_top = false;
+  int64_t cand_total = 0;
   int capmax = 1;
   for (int i = 0; i < nn; ++i) {
     const AcaDesc& d = descs[i];
@@ -314,8 +309,6 @@ static int run_aca2(bgp_hodlr* h, const std::vector<AcaDesc>& descs, std::vector
     for (int c = 0; c < a.n_rchunks; ++c) rchunk_node.push_back(i);
     a.bmax = std::min(A2_BMAX, d.n_rows);
     a.cand_off = cand_total; cand_total += a.bmax;
-    a.is_top = (dist_top && h->nodes[d.pre_id].top) ? 1 : 0;
-    if (a.is_top) top_cand_total = cand_total;
     capmax = std::max(capmax, d.cap);
   }
   const int ncc = (int)cchunk_node.size(), nrc = (int)rchunk_node.size();
@@ -340,9 +333,7 @@ static int run_aca2(bgp_hodlr* h, const std::vector<AcaDesc>& descs, std::vector
     BGP_TRY(h->d_vmax.reserve((size_t)ncc * A2_NGROUP, s));
     BGP_TRY(h->d_cand_xu.reserve((size_t)cand_total, s));
   }
-  BGP_TRY(h->d_nactive.reserve(2, s));
-  int n_top = 0;
-  for (int i = 0; i < nn; ++i) n_top += hn[i].is_top;
+  BGP_TRY(h->d_nactive.reserve(1, s));
   BGP_TRY(h->d_stats.reserve(4, s));
   int64_t work_cap = 0;
   // items per chunk: batches of up to 256 live candidates are cut into blocks of A2_CG, larger ones into A2_CG * A2_ITEM_CB
@@ -373,8 +364,6 @@ static int run_aca2(bgp_hodlr* h, const std::vector<AcaDesc>& descs, std::vector
   a.cand_L = h->d_cand_L.p; a.cand_next = h->d_cand_next.p; a.cand_live = h->d_cand_live.p; a.node_box = h->d_node_box.p;
   a.capmax = capmax; a.n_active = h->d_nactive.p; a.stats = h->d_stats.p;
   a.work = h->d_work.p; a.work_count = h->d_work_count.p; a.work_cursor = h->d_work_count.p + 2; a.work_cap = (int)work_cap; a.iter_ptr = h->d_iter.p;
-  a.shard_rank = dist_top ? h->opts.shard_rank : 0; a.shard_count = dist_top ? h->opts.shard_count : 1;
-  if (dist_top) BGP_CUDA(cudaMemcpyAsync(h->d_nactive.p + 1, &n_top, sizeof(int), cudaMemcpyHostToDevice, s));
   // (the attribute is per device / context: set it on every call, it is cheap)
   cudaFuncSetAttribute(a2_init_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(A2NodeSmem));
     cudaFuncSetAttribute(a2_decide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(A2NodeSmem));
@@ -382,8 +371,6 @@ static int run_aca2(bgp_hodlr* h, const std::vector<AcaDesc>& descs, std::vector
   a2_init_kernel<<<nn, A2_NODE_THREADS, sizeof(A2NodeSmem), s>>>(a);
   BGP_LAUNCH_CHECK();
   int active = nn, iters = 0;
-  int eval_minb = A2_EVAL_MINB_DEFAULT;
-  if (const char* e = getenv("BGP_EVAL_MINB")) eval_minb = atoi(e) == 3 ? 3 : 2;
   const int eval_grid = num_sms() * 6;  // persistent CTAs over the work list (2-3 resident per SM, a few rounds)
   // One lock-step iteration = eval -> decide -> vrow -> pivot -> vnorm|ucol -> finish -> tick.
   auto launch_iteration = [&](cudaStream_t st, cudaGraphConditionalHandle hnd, int use_hnd, int it_prof) -> int {
@@ -391,15 +378,14 @@ static int run_aca2(bgp_hodlr* h, const std::vector<AcaDesc>& descs, std::vector
       if (it_prof < 0) return BGP_OK;
       const size_t need = (size_t)7 * (it_prof + 1);
       while (h->prof_events.size() < need) {
-        cudaEvent_t e;
-        BGP_CUDA(cudaEventCreate(&e));
-        h->prof_events.push_back(e);
+        h->prof_events.emplace_back();
+        BGP_TRY(h->prof_events.back().create());
       }
       BGP_CUDA(cudaEventRecord(h->prof_events[(size_t)7 * it_prof + slot], st));
       return BGP_OK;
     };
     BGP_TRY(mark(0));
-    a2_eval_launch(h->prog.shape, dim3(eval_grid), st, a, eval_minb);
+    a2_eval_launch(h->prog.shape, dim3(eval_grid), st, a);
     BGP_LAUNCH_CHECK();
     BGP_TRY(mark(1));
     a2_decide_kernel<<<nn, A2_NODE_THREADS, sizeof(A2NodeSmem), st>>>(a);
@@ -428,49 +414,46 @@ static int run_aca2(bgp_hodlr* h, const std::vector<AcaDesc>& descs, std::vector
     // calls compute() with the same shapes and buffers over and over.
     AcaGraphKey key;
     memset(&key, 0, sizeof(key));
-    key.a = a; key.nn = nn; key.ncc = ncc; key.nrc = nrc; key.shape = h->prog.shape; key.grid = eval_grid * 4 + eval_minb;
-    if (!h->aca_exec || memcmp(&key, &h->aca_key, sizeof(key)) != 0) {
-      if (h->aca_exec) { cudaGraphExecDestroy(h->aca_exec); h->aca_exec = nullptr; }
-      if (h->aca_graph) { cudaGraphDestroy(h->aca_graph); h->aca_graph = nullptr; }
-      BGP_CUDA(cudaGraphCreate(&h->aca_graph, 0));
+    key.a = a; key.nn = nn; key.ncc = ncc; key.nrc = nrc; key.shape = h->prog.shape; key.grid = eval_grid;
+    if (!h->aca.exec || memcmp(&key, &h->aca.key, sizeof(key)) != 0) {
+      h->aca.reset();
+      BGP_CUDA(cudaGraphCreate(&h->aca.graph, 0));
       cudaGraphConditionalHandle hnd;
-      BGP_CUDA(cudaGraphConditionalHandleCreate(&hnd, h->aca_graph, 1, cudaGraphCondAssignDefault));
+      BGP_CUDA(cudaGraphConditionalHandleCreate(&hnd, h->aca.graph, 1, cudaGraphCondAssignDefault));
       cudaGraphNodeParams cp = {};
       cp.type = cudaGraphNodeTypeConditional;
       cp.conditional.handle = hnd;
       cp.conditional.type = cudaGraphCondTypeWhile;
       cp.conditional.size = 1;
       cudaGraphNode_t wnode;
-      BGP_CUDA(cudaGraphAddNode(&wnode, h->aca_graph, nullptr, 0, &cp));
+      BGP_CUDA(cudaGraphAddNode(&wnode, h->aca.graph, nullptr, 0, &cp));
       cudaGraph_t body = cp.conditional.phGraph_out[0];
-      if (!h->sC) BGP_CUDA(cudaStreamCreateWithFlags(&h->sC, cudaStreamNonBlocking));
+      BGP_TRY(h->sC.create());
       BGP_CUDA(cudaStreamBeginCaptureToGraph(h->sC, body, nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed));
       const int rc = launch_iteration(h->sC, hnd, 1, -1);
       cudaGraph_t captured = nullptr;
       const cudaError_t ce = cudaStreamEndCapture(h->sC, &captured);
       if (rc != BGP_OK) return rc;
       if (ce != cudaSuccess) { set_error("ACA graph capture failed: %s", cudaGetErrorString(ce)); return BGP_ERR_CUDA; }
-      BGP_CUDA(cudaGraphInstantiate(&h->aca_exec, h->aca_graph, 0));
-      h->aca_key = key;
+      BGP_CUDA(cudaGraphInstantiate(&h->aca.exec, h->aca.graph, 0));
+      h->aca.key = key;
     }
-    BGP_CUDA(cudaGraphLaunch(h->aca_exec, s));
-    int it_host = 0, act2[2] = {0, 0};
+    BGP_CUDA(cudaGraphLaunch(h->aca.exec, s));
+    int it_host = 0;
     BGP_CUDA(cudaMemcpyAsync(&it_host, h->d_iter.p, sizeof(int), cudaMemcpyDeviceToHost, s));
-    BGP_CUDA(cudaMemcpyAsync(act2, h->d_nactive.p, sizeof(int) * 2, cudaMemcpyDeviceToHost, s));
+    BGP_CUDA(cudaMemcpyAsync(&active, h->d_nactive.p, sizeof(int), cudaMemcpyDeviceToHost, s));
     BGP_CUDA(cudaStreamSynchronize(s));
     iters = it_host;
     g_launches.fetch_add((uint64_t)7 * (uint64_t)std::max(iters - 1, 0), std::memory_order_relaxed);  // the capture counted one iteration
-    if (act2[0] > 0) { set_error("ACA did not terminate"); return BGP_ERR_CUDA; }
+    if (active > 0) { set_error("ACA did not terminate"); return BGP_ERR_CUDA; }
   } else {
     while (active > 0) {
       for (int rep = 0; rep < 8; ++rep) {
         BGP_TRY(launch_iteration(s, 0, 0, h->profile ? iters : -1));
         iters++;
       }
-      int act2[2] = {0, 0};
-      BGP_CUDA(cudaMemcpyAsync(act2, h->d_nactive.p, sizeof(int) * 2, cudaMemcpyDeviceToHost, s));
+      BGP_CUDA(cudaMemcpyAsync(&active, h->d_nactive.p, sizeof(int), cudaMemcpyDeviceToHost, s));
       BGP_CUDA(cudaStreamSynchronize(s));
-      active = act2[0];
       if (iters > (1 << 22)) { set_error("ACA did not terminate"); return BGP_ERR_CUDA; }
     }
   }
@@ -508,6 +491,36 @@ static int run_aca2(bgp_hodlr* h, const std::vector<AcaDesc>& descs, std::vector
     houts[descs[i].node] = o;
   }
   return BGP_OK;
+}
+
+// log-determinant = sum of the leaf and node log-dets of this process.  A sharded run factors the nodes above the cut on
+// every rank but counts them on shard 0 only, so that the sum over the shards counts each node once.
+static int sum_log_det(bgp_hodlr* h, cudaStream_t s, double* out) {
+  const int nl = (int)h->leaves.size(), nlev = (int)h->levels.size();
+  int ndesc = 0;
+  for (auto& L : h->levels) ndesc += (int)L.nodes.size();
+  std::vector<double> ld_leaf(nl), ld_node(ndesc);
+  if (nl) BGP_CUDA(cudaMemcpyAsync(ld_leaf.data(), h->d_leaf_logdet.p, sizeof(double) * nl, cudaMemcpyDeviceToHost, s));
+  if (ndesc) BGP_CUDA(cudaMemcpyAsync(ld_node.data(), h->d_node_logdet.p, sizeof(double) * ndesc, cudaMemcpyDeviceToHost, s));
+  BGP_CUDA(cudaStreamSynchronize(s));
+  const int cut = std::min(h->cut_depth, nlev);
+  double ld = 0.0;
+  for (double v : ld_leaf) ld += v;
+  for (int l = 0; l < nlev; ++l) {
+    const LevelInfo& L = h->levels[l];
+    if (l < cut && h->opts.shard_rank != 0) continue;
+    for (size_t i = 0; i < L.nodes.size(); ++i) ld += ld_node[L.desc_off + i];
+  }
+  *out = ld;
+  return BGP_OK;
+}
+
+static void record_compute_timing(bgp_hodlr* h) {
+  float ms = 0;
+  cudaEventElapsedTime(&ms, h->ev[0], h->ev[1]); h->t_ms[0] = ms;
+  cudaEventElapsedTime(&ms, h->ev[0], h->ev[2]); h->t_ms[1] = ms;
+  cudaEventElapsedTime(&ms, h->ev[6], h->ev[3]); h->t_ms[2] = ms;  // panel finalisation + leaf solves + level sweeps only
+  cudaEventElapsedTime(&ms, h->ev[0], h->ev[3]); h->t_ms[3] = ms;
 }
 
 static int hodlr_compute_dev_impl(bgp_hodlr* h, const bgp_kernel_spec_t* spec, const double* x_dev, int64_t n,
@@ -563,10 +576,9 @@ static int hodlr_compute_dev_impl(bgp_hodlr* h, const bgp_kernel_spec_t* spec, c
   h->levels.assign(max_depth + 1, LevelInfo());
   for (size_t i = 0; i < h->nodes.size(); ++i) {
     HNode& nd = h->nodes[i];
-    if (nd.is_leaf) { if (nd.owned) { nd.slot = (int)h->leaves.size(); h->leaves.push_back((int)i); } continue; }
+    if (nd.is_leaf) { if (nd.owned) h->leaves.push_back((int)i); continue; }
     if (!(nd.owned || nd.top)) continue;
     LevelInfo& L = h->levels[nd.depth];
-    nd.slot = (int)L.nodes.size();
     L.nodes.push_back((int)i);
     L.max_half = std::max(L.max_half, nd.size - nd.half);
   }
@@ -642,7 +654,6 @@ static int hodlr_compute_dev_impl(bgp_hodlr* h, const bgp_kernel_spec_t* spec, c
     int vcols_set[2] = {0, 0};
     for (auto& L : h->levels) { L.vcol = vcols_set[L.set]; vcols_set[L.set] += L.cap; }
     h->top.vcols = vcols_set[0]; h->loc.vcols = vcols_set[1];
-    h->vcols = vcols_set[0] + vcols_set[1];
     hdesc.clear(); desc_node.clear();
     h->piv_off.assign(h->nodes.size(), -1);
     idx_total = 0; piv_total = 0; nint = 0;
@@ -665,7 +676,7 @@ static int hodlr_compute_dev_impl(bgp_hodlr* h, const bgp_kernel_spec_t* spec, c
     if (o.rng_mode == BGP_RNG_REFERENCE) std::sort(order.begin(), order.end(), [&](int a, int b) { return hdesc[a].pre_id < hdesc[b].pre_id; });
     else std::stable_sort(order.begin(), order.end(), [&](int a, int b) {
       const int ta = h->nodes[hdesc[a].pre_id].top, tb = h->nodes[hdesc[b].pre_id].top;
-      if (ta != tb) return ta > tb;  // nodes above the shard cut first (contiguous candidate range for the all-reduce)
+      if (ta != tb) return ta > tb;  // nodes above the shard cut first
       return hdesc[a].n_rows > hdesc[b].n_rows;
     });
     std::vector<AcaDesc> hdesc_sorted(nint);
@@ -709,7 +720,7 @@ static int hodlr_compute_dev_impl(bgp_hodlr* h, const bgp_kernel_spec_t* spec, c
       cudaFuncSetAttribute(aca_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
       if (smem > 200 * 1024) { set_error("rank capacity %d too large", maxcap); return BGP_ERR_RANK_CAPACITY; }
       aca_kernel<<<nint, ACA_THREADS, smem, sB>>>(h->d_prog.p, h->d_x.p, h->d_aca.p, nint, h->loc.vbase(), h->loc.ld, o.tol, (uint32_t)o.seed,
-                                                  o.rng_mode, h->d_idx.p, h->d_piv_rows.p, h->d_piv_cols.p, h->d_aca_out.p,
+                                                  h->d_idx.p, h->d_piv_rows.p, h->d_piv_cols.p, h->d_aca_out.p,
                                                   h->d_ticket.p, h->d_chain_state.p, h->d_chain_done.p, o.exhaust_mode);
       BGP_LAUNCH_CHECK();
       BGP_CUDA(cudaMemcpyAsync(houts.data(), h->d_aca_out.p, sizeof(AcaOut) * nint, cudaMemcpyDeviceToHost, sB));
@@ -768,7 +779,6 @@ static int hodlr_compute_dev_impl(bgp_hodlr* h, const bgp_kernel_spec_t* spec, c
   }
   h->top.ucols = rtot_set[0]; h->loc.ucols = rtot_set[1];
   const int rtot = rtot_set[0] + rtot_set[1];
-  h->rtot = rtot;
   // per-depth number of LOCAL ancestor columns a leaf (or node) at that depth sees (levels above the cut live in the top
   // panel set and receive this shard's sub-tree inverse in a separate pass, below)
   std::vector<int> ncols_by_depth(max_depth + 2, h->loc.ucols);
@@ -825,25 +835,9 @@ static int hodlr_compute_dev_impl(bgp_hodlr* h, const bgp_kernel_spec_t* spec, c
     return BGP_OK;
   }
 
-  // ---- log-det ----
-  std::vector<double> ld_leaf(nl), ld_node(ndesc);
-  if (nl) BGP_CUDA(cudaMemcpyAsync(ld_leaf.data(), h->d_leaf_logdet.p, sizeof(double) * nl, cudaMemcpyDeviceToHost, sA));
-  if (ndesc) BGP_CUDA(cudaMemcpyAsync(ld_node.data(), h->d_node_logdet.p, sizeof(double) * ndesc, cudaMemcpyDeviceToHost, sA));
-  if (nint) {
-    h->h_piv_rows.resize(piv_total); h->h_piv_cols.resize(piv_total);
-  }
-  BGP_CUDA(cudaStreamSynchronize(sA));
-  double ld = 0.0;
-  for (double v : ld_leaf) ld += v;
-  for (double v : ld_node) ld += v;
-  h->log_det = ld;
+  BGP_TRY(sum_log_det(h, sA, &h->log_det));
   h->computed = true;
-
-  float ms = 0;
-  cudaEventElapsedTime(&ms, h->ev[0], h->ev[1]); h->t_ms[0] = ms;
-  cudaEventElapsedTime(&ms, h->ev[0], h->ev[2]); h->t_ms[1] = ms;
-  cudaEventElapsedTime(&ms, h->ev[6], h->ev[3]); h->t_ms[2] = ms;  // panel finalisation + leaf solves + level sweeps only
-  cudaEventElapsedTime(&ms, h->ev[0], h->ev[3]); h->t_ms[3] = ms;
+  record_compute_timing(h);
 
   // algorithmic work (SURVEY.md §8d)
   {
@@ -905,12 +899,6 @@ static int hodlr_solve_dev(bgp_hodlr* h, double* b, int64_t nrhs, int64_t ldb, c
   return BGP_OK;
 }
 
-static int64_t top_cols(const bgp_hodlr_t* h) {
-  const int cut = std::min<int>(h->cut_depth, (int)h->levels.size());
-  (void)cut;
-  return h->top.ucols;
-}
-
 // Gram / LU / log-det / update of the nodes above the shard cut (every rank does all of them: they are tiny), then the
 // log-determinant: owned leaves + owned nodes, the top nodes counted once (by shard 0); with `allreduce` the partial sums
 // are added over the ranks on the device (one double), otherwise log_det stays PARTIAL and the host sums over shards.
@@ -922,20 +910,8 @@ static int hodlr_finish_top_impl(bgp_hodlr* h, bool allreduce) {
     const LevelInfo& L = h->levels[l];
     BGP_TRY(launch_level(h, L, h->top.U.p, h->n, L.ucol + L.r, L.ucol, 1, 0, L.ucol, s));
   }
-  const int nl = (int)h->leaves.size();
-  int ndesc = 0;
-  for (auto& L : h->levels) ndesc += (int)L.nodes.size();
-  std::vector<double> ld_leaf(nl), ld_node(ndesc);
-  if (nl) BGP_CUDA(cudaMemcpyAsync(ld_leaf.data(), h->d_leaf_logdet.p, sizeof(double) * nl, cudaMemcpyDeviceToHost, s));
-  if (ndesc) BGP_CUDA(cudaMemcpyAsync(ld_node.data(), h->d_node_logdet.p, sizeof(double) * ndesc, cudaMemcpyDeviceToHost, s));
-  BGP_CUDA(cudaStreamSynchronize(s));
   double ld = 0.0;
-  for (double v : ld_leaf) ld += v;
-  for (int l = 0; l < nlev; ++l) {
-    const LevelInfo& L = h->levels[l];
-    if (l < cut && h->opts.shard_rank != 0) continue;
-    for (size_t i = 0; i < L.nodes.size(); ++i) ld += ld_node[L.desc_off + i];
-  }
+  BGP_TRY(sum_log_det(h, s, &ld));
   if (allreduce) {
     BGP_CUDA(cudaMemcpyAsync(h->d_scalar.p, &ld, sizeof(double), cudaMemcpyHostToDevice, s));
     BGP_TRY(comm_allreduce_sum_f64(h->d_scalar.p, 1, s));
@@ -950,13 +926,9 @@ static int hodlr_finish_top_impl(bgp_hodlr* h, bool allreduce) {
 // sharded compute with the library's communicator: all-gather of the locally solved rows of the top-level factor panel
 // (the ONE data-path collective of compute(), SURVEY.md §8e), then the top nodes, then the log-det all-reduce.
 static int hodlr_exchange_finish(bgp_hodlr* h) {
-  BGP_TRY(exchange_rows(h, h->top.U.p, h->n, top_cols(h), h->sA));
+  BGP_TRY(exchange_rows(h, h->top.U.p, h->n, h->top.ucols, h->sA));
   BGP_TRY(hodlr_finish_top_impl(h, true));
-  float ms = 0;
-  cudaEventElapsedTime(&ms, h->ev[0], h->ev[1]); h->t_ms[0] = ms;
-  cudaEventElapsedTime(&ms, h->ev[0], h->ev[2]); h->t_ms[1] = ms;
-  cudaEventElapsedTime(&ms, h->ev[6], h->ev[3]); h->t_ms[2] = ms;
-  cudaEventElapsedTime(&ms, h->ev[0], h->ev[3]); h->t_ms[3] = ms;
+  record_compute_timing(h);
   return BGP_OK;
 }
 
@@ -977,30 +949,6 @@ int bgp_hodlr_create(bgp_hodlr_t** out) {
 
 void bgp_hodlr_destroy(bgp_hodlr_t* h) {
   if (!h) return;
-  if (h->sA) {
-    cudaStreamSynchronize(h->sA); cudaStreamSynchronize(h->sB);
-  }
-  // release buffers while the streams are still alive
-  h->d_prog.release(); h->d_x.release(); h->d_yerr.release(); h->d_diag.release(); h->d_L.release();
-  h->d_leaf_logdet.release(); h->d_node_logdet.release(); h->top.V.release(); h->top.U.release(); h->loc.V.release(); h->loc.U.release(); h->d_S.release();
-  h->d_W.release(); h->d_scalar.release(); h->d_rhs.release(); h->d_leaves.release(); h->d_aca.release();
-  h->d_aca_out.release(); h->d_nodes.release(); h->d_idx.release(); h->d_piv_rows.release(); h->d_piv_cols.release();
-  h->lu_ws.d_nodes.release(); h->lu_ws.d_trsm.release(); h->lu_ws.d_gemm.release(); h->d_gram_desc.release(); h->d_upd_desc.release();
-  h->d_ticket.release(); h->d_chain_done.release(); h->d_ncols_by_depth.release(); h->d_chain_state.release();
-  h->d_a2nodes.release(); h->d_a2states.release(); h->d_a2rngs.release(); h->d_epart.release(); h->d_cand.release(); h->d_cand_k.release();
-  h->d_cand_words.release(); h->d_cand_L.release(); h->d_cand_next.release(); h->d_cand_live.release(); h->d_node_box.release(); h->d_cand_xu.release(); h->d_cchunk_node.release(); h->d_rchunk_node.release(); h->d_nactive.release();
-  h->d_inv.release(); h->d_gscratch.release(); h->d_which.release(); h->d_xsend.release(); h->d_xrecv.release();
-  h->d_vpart.release(); h->d_upart.release(); h->d_vmax.release(); h->d_cmax.release(); h->d_stats.release(); h->d_work.release(); h->d_work_count.release();
-  for (cudaEvent_t e : h->prof_events) cudaEventDestroy(e);
-  h->d_iter.release();
-  if (h->aca_exec) cudaGraphExecDestroy(h->aca_exec);
-  if (h->aca_graph) cudaGraphDestroy(h->aca_graph);
-  if (h->sC) cudaStreamDestroy(h->sC);
-  if (h->sA) {
-    cudaStreamSynchronize(h->sA); cudaStreamSynchronize(h->sB);
-    for (int i = 0; i < 8; ++i) cudaEventDestroy(h->ev[i]);
-    cudaStreamDestroy(h->sA); cudaStreamDestroy(h->sB);
-  }
   delete h;
 }
 
@@ -1222,10 +1170,8 @@ int bgp_selftest_gemm(int32_t a_kcontig, int32_t b_kcontig, int32_t m, int32_t n
 // ---- multi-GPU exchange (SURVEY.md §8e) -----------------------------------------------------------------------
 int bgp_hodlr_top_panel(bgp_hodlr_t* h, double** ptr_dev, int64_t* row0, int64_t* rows, int64_t* cols, int64_t* ld) {
   if (!h) { set_error("null handle"); return BGP_ERR_INVALID; }
-  const int cut = std::min<int>(h->cut_depth, (int)h->levels.size());
   *ptr_dev = h->top.U.p;
   *row0 = h->row0; *rows = h->nloc;
-  (void)cut;
   *cols = h->top.ucols;
   *ld = h->n;
   return BGP_OK;
@@ -1240,7 +1186,7 @@ int bgp_hodlr_shard_rows(const bgp_hodlr_t* h, int32_t s, int64_t* row0, int64_t
 
 int bgp_hodlr_export_top(bgp_hodlr_t* h, double* buf_dev, int64_t rows_pad) {
   if (!h) { set_error("null handle"); return BGP_ERR_INVALID; }
-  const int64_t cols = top_cols(h);
+  const int64_t cols = h->top.ucols;
   if (cols == 0 || h->nloc == 0) return BGP_OK;
   if (rows_pad < h->nloc) { set_error("rows_pad too small"); return BGP_ERR_INVALID; }
   pack_rows_kernel<<<1184, 256, 0, h->sA>>>(h->top.U.p, h->n, h->row0, h->nloc, cols, buf_dev, rows_pad);
@@ -1251,7 +1197,7 @@ int bgp_hodlr_export_top(bgp_hodlr_t* h, double* buf_dev, int64_t rows_pad) {
 
 int bgp_hodlr_import_top(bgp_hodlr_t* h, const double* all_buf_dev, int64_t rows_pad) {
   if (!h) { set_error("null handle"); return BGP_ERR_INVALID; }
-  const int64_t cols = top_cols(h);
+  const int64_t cols = h->top.ucols;
   if (cols == 0) return BGP_OK;
   for (size_t s = 0; s < h->shard_rows.size(); ++s) {
     if ((int)s == h->opts.shard_rank) continue;  // own rows are already in place

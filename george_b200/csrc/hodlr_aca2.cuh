@@ -15,7 +15,8 @@
 //       leave the kernel, through atomicMax) -> decide (first usable candidate; RNG / row list committed to that draw)
 //       -> vrow (winning row's residual + chunk arg-max) -> pivot -> vnorm || ucol (one launch) -> finish (stopping
 //       rule, next candidates).  The host reads one "active nodes" counter every 8 iterations.
-//   * sharded runs split the scan of the nodes above the cut across ranks and MAX-all-reduce the maxima (comm.cu).
+//   * sharded runs: every rank scans the nodes above the cut itself.  With bound culling and one-candidate batches the
+//     scans are cheap, and a collective inside the lock-step loop would put a latency on every step.
 #pragma once
 
 #include "hodlr_kernels.cuh"
@@ -30,7 +31,6 @@ constexpr int A2_EPT = A2_CHUNK / A2_THREADS;  // elements per thread
 constexpr int A2_CG = 4;          // candidates evaluated together (register blocking)
 constexpr int A2_ITEM_CB = 8;      // candidate blocks (of A2_CG rows) per eval work item
 constexpr int A2_BMAX = 8192;     // max speculative candidates per iteration (bounded by the per-node CTA's shared memory)
-constexpr int A2_EVAL_MINB_DEFAULT = 3;  // see a2_eval_kernel (BGP_EVAL_MINB=3 selects the other build at run time)
 constexpr int A2_BGROW = 8;       // batch growth after a fully rejected batch: 4, 32, 256, 2048, 8192
 constexpr int A2_NSUB = 4;        // the residual kernels (vrow / ucol / vnorm) split a chunk into sub-chunks of A2_THREADS
 constexpr int A2_GROUP = A2_CHUNK / (A2_THREADS / 32);  // 128 columns: what one warp of a2_eval sweeps (bound granularity)
@@ -44,7 +44,7 @@ struct A2Node {  // static description
   int row0, n_rows, col0, n_cols;
   int vcol, cap, pre_id, node;
   int cchunk0, n_cchunks, rchunk0, n_rchunks;
-  int bmax, is_top;  // is_top: node above the shard cut, its candidate scan is split across ranks by column chunk
+  int bmax;
   int64_t idx_off, piv_off, cand_off;
   double* vbase;   // column 0 of this node's level in ITS factor panel, addressed by GLOBAL row index: the panel of a level
                    // owned by one shard holds only that shard's rows (leading dimension ld = rows of the shard) and vbase
@@ -176,7 +176,6 @@ struct A2Args {
   int* work_cursor;    // [2] next (item, group) unit of the buffer being consumed (a2_eval pulls work dynamically)
   int work_cap;
   int* iter_ptr;       // device counter: lock-step iteration number (selects the buffers); advanced by a2_tick_kernel
-  int shard_rank, shard_count;  // multi-GPU: top nodes' column chunks are dealt round-robin to the ranks
   unsigned long long* stats;  // [0] candidate-row entries verified (pairs), [1] residual-update FMAs executed, [2] candidates,
                               // [3] entries actually evaluated by a2_eval (the rest were bounded < 1e-14 without evaluation)
 };
@@ -393,8 +392,7 @@ __device__ inline void a2_generate(const A2Args& a, A2State& st, A2NodeSmem& S, 
     }
   }
   __syncthreads();
-  // publish the evaluation work of the NEXT eval launch: one item = (column chunk, up to A2_CG * A2_ITEM_CB live candidates).
-  // In a sharded run the chunks of a node above the cut are dealt round-robin to the ranks.
+  // publish the evaluation work of the NEXT eval launch: one item = (column chunk, up to A2_CG * A2_ITEM_CB live candidates)
   {
     int n_live = S.n_live;
     const bool defer = (B == 1 && n_live == 1);
@@ -403,10 +401,7 @@ __device__ inline void a2_generate(const A2Args& a, A2State& st, A2NodeSmem& S, 
     // few live candidates: one block of A2_CG per item, so that the sweep has no sequential depth inside an item
     const int ipc = (n_live <= 256) ? A2_CG : A2_CG * A2_ITEM_CB;
     const int per_chunk = (n_live + ipc - 1) / ipc;
-    int my_chunks = nd.n_cchunks;
-    const bool split = nd.is_top && a.shard_count > 1;
-    if (split) my_chunks = (nd.n_cchunks - a.shard_rank + a.shard_count - 1) / a.shard_count;
-    const int n_items = my_chunks * per_chunk;
+    const int n_items = nd.n_cchunks * per_chunk;
     int4* work_next = a.work + (int64_t)nb * a.work_cap;
     __syncthreads();
     if (threadIdx.x == 0) {
@@ -417,9 +412,8 @@ __device__ inline void a2_generate(const A2Args& a, A2State& st, A2NodeSmem& S, 
     const int base = S.flag;
     for (int t = threadIdx.x; t < n_items; t += blockDim.x) {
       const int ci = t / per_chunk, pi = t % per_chunk;
-      const int lc = split ? (a.shard_rank + ci * a.shard_count) : ci;
       const int c0 = pi * ipc;
-      if (base + t < a.work_cap) work_next[base + t] = make_int4(nd.cchunk0 + lc, c0, min(ipc, n_live - c0), nid);
+      if (base + t < a.work_cap) work_next[base + t] = make_int4(nd.cchunk0 + ci, c0, min(ipc, n_live - c0), nid);
     }
   }
   __syncthreads();
@@ -443,7 +437,7 @@ __global__ void __launch_bounds__(A2_NODE_THREADS) a2_init_kernel(A2Args a) {
   mt_copy(a.rngs + 2 * (int64_t)nid, &S.rng);  // committed = state before the speculative draws
   __syncthreads();
   if (nd.cap <= 0) {
-    if (threadIdx.x == 0) { st.status = 1; st.phase = A2_DONE; st.active = 0; { atomicSub(a.n_active, 1); if (nd.is_top) atomicSub(a.n_active + 1, 1); } }
+    if (threadIdx.x == 0) { st.status = 1; st.phase = A2_DONE; st.active = 0; atomicSub(a.n_active, 1); }
     return;
   }
   // bounding interval of the node's columns (candidate-level bound culling; 1-D programs with a distance bound only)
@@ -590,11 +584,11 @@ __device__ __forceinline__ void a2_eval_body(const A2Args& a, const A2Node& nd, 
   }
 }
 
-// one instantiation per program shape: the specialised ones carry no interpreter and need far fewer registers
-// MINB = CTAs per SM the register allocation is made for: 2 -> 128 registers, no spills; 3 -> 80 registers and a few
-// spilled temporaries of the software exp / sqrt chains, but 24 instead of 16 warps per SM to hide their latency
-template <int SHAPE, int MINB>
-__global__ void __launch_bounds__(A2_THREADS, MINB) a2_eval_kernel(A2Args a) {
+// one instantiation per program shape: the specialised ones carry no interpreter and need far fewer registers.
+// Register allocation for 3 CTAs per SM on the specialised shapes (80 registers and a few spilled temporaries of the
+// software exp / sqrt chains, but 24 instead of 16 warps per SM to hide their latency), 2 on the interpreter (128, no spills)
+template <int SHAPE>
+__global__ void __launch_bounds__(A2_THREADS, SHAPE == BGP_SHAPE_GENERIC ? 2 : 3) a2_eval_kernel(A2Args a) {
   __shared__ DevProgram P;
   // persistent CTAs sweep the work list published by the node kernels of the previous step: perfectly balanced over
   // the chip whatever mix of nodes is still active, and no empty CTAs
@@ -628,12 +622,8 @@ __global__ void __launch_bounds__(A2_THREADS, MINB) a2_eval_kernel(A2Args a) {
   }
   if ((threadIdx.x & 31) == 0 && n_eval) { atomicAdd(a.stats + 3, n_eval); atomicAdd(a.stats + 1, n_fma); }
 }
-inline void a2_eval_launch(int shape, dim3 grid, cudaStream_t s, const A2Args& a, int minb) {
-  if (minb == 3 && shape != BGP_SHAPE_GENERIC) {
-    BGP_SHAPE_SWITCH(shape, (a2_eval_kernel<SHAPE, (SHAPE == BGP_SHAPE_GENERIC ? 2 : 3)><<<grid, A2_THREADS, 0, s>>>(a)));
-  } else {
-    BGP_SHAPE_SWITCH(shape, (a2_eval_kernel<SHAPE, 2><<<grid, A2_THREADS, 0, s>>>(a)));
-  }
+inline void a2_eval_launch(int shape, dim3 grid, cudaStream_t s, const A2Args& a) {
+  BGP_SHAPE_SWITCH(shape, (a2_eval_kernel<SHAPE><<<grid, A2_THREADS, 0, s>>>(a)));
 }
 
 // ---- decide: first usable candidate wins; commit the RNG / index list up to it ----------------------------------
@@ -719,7 +709,7 @@ __global__ void __launch_bounds__(A2_NODE_THREADS) a2_decide_kernel(A2Args a) {
     if (st.n_index == 0) {
       st.fallback = 1;  // rows exhausted (hodlr.h:161); dense fill (if requested) happens after the loop
       st.phase = A2_DONE; st.active = 0;
-      { atomicSub(a.n_active, 1); if (nd.is_top) atomicSub(a.n_active + 1, 1); }
+      atomicSub(a.n_active, 1);
     }
   }
   __syncthreads();
@@ -986,7 +976,7 @@ __global__ void __launch_bounds__(A2_NODE_THREADS) a2_finish_kernel(A2Args a) {
       if (st.n_index == 0) {
         st.fallback = 1;
         st.phase = A2_DONE; st.active = 0;
-        { atomicSub(a.n_active, 1); if (nd.is_top) atomicSub(a.n_active + 1, 1); }
+        atomicSub(a.n_active, 1);
       } else {
         st.phase = A2_SELECT;
       }
@@ -1041,7 +1031,7 @@ __global__ void __launch_bounds__(A2_NODE_THREADS) a2_finish_kernel(A2Args a) {
     }
     if (done) {
       st.phase = A2_DONE; st.active = 0;
-      { atomicSub(a.n_active, 1); if (nd.is_top) atomicSub(a.n_active + 1, 1); }
+      atomicSub(a.n_active, 1);
     } else {
       st.phase = A2_SELECT;
     }

@@ -209,8 +209,7 @@ __global__ void __launch_bounds__(LEAF_THREADS) leaf_build_factor_kernel(const D
 // staged in shared memory and all threads cooperate on the substitutions.
 // ---------------------------------------------------------------------------------------------------------------
 constexpr int LS_THREADS = 256;
-constexpr int LS_COLS = 8;        // right-hand sides per CTA of the narrow instantiation (a solve: 1 .. 8 columns)
-constexpr int LS_COLS_WIDE = 32;  // ... of the wide one (BGP_LEAF_COLS=32; measured slower than four narrow groups, see hodlr.cu)
+constexpr int LS_COLS = 8;        // right-hand sides per CTA (32 measured slower for the up-sweep: DESIGN.md §8.3)
 constexpr int LS_NB = 32;         // diagonal block
 
 // Blocked substitution: per 32-column block of L, (a) the 32 x 32 diagonal block is staged in shared memory and each
@@ -382,13 +381,13 @@ __device__ __forceinline__ double block_max_signed(double v, double* red) {  // 
   return warp_max(t);
 }
 
-// rng_mode BGP_RNG_REFERENCE: CTAs take tickets in pre-order and chain the single mt19937 through `chain_state`
+// rng_mode = reference: CTAs take tickets in pre-order and chain the single mt19937 through `chain_state`
 // (624 words + index) guarded by `chain_done[k]` flags — the pre-order dependence of hodlr.h:35,58-61 made explicit.
 __global__ void __launch_bounds__(ACA_THREADS) aca_kernel(const DevProgram* __restrict__ gprog,
                                                           const double* __restrict__ x,
                                                           const AcaDesc* __restrict__ descs, int n_desc,
                                                           double* __restrict__ Vp, int64_t ld, double tol,
-                                                          uint32_t seed, int rng_mode, int* __restrict__ idx_ws,
+                                                          uint32_t seed, int* __restrict__ idx_ws,
                                                           int* __restrict__ piv_rows, int* __restrict__ piv_cols,
                                                           AcaOut* __restrict__ outs, int* __restrict__ ticket,
                                                           uint32_t* chain_state, volatile int* chain_done,
@@ -414,17 +413,13 @@ __global__ void __launch_bounds__(ACA_THREADS) aca_kernel(const DevProgram* __re
 
   for (int n = threadIdx.x; n < n_rows; n += blockDim.x) index[n] = n;
   if (threadIdx.x == 0) {
-    if (rng_mode == BGP_RNG_REFERENCE) {
-      if (tk > 0) {
-        while (chain_done[tk - 1] == 0) __nanosleep(200);
-        __threadfence();
-        for (int i = 0; i < 624; ++i) S->rng.mt[i] = chain_state[i];
-        S->rng.idx = (int)chain_state[624];
-      } else {
-        mt_seed(S->rng, seed);
-      }
+    if (tk > 0) {
+      while (chain_done[tk - 1] == 0) __nanosleep(200);
+      __threadfence();
+      for (int i = 0; i < 624; ++i) S->rng.mt[i] = chain_state[i];
+      S->rng.idx = (int)chain_state[624];
     } else {
-      mt_seed(S->rng, node_seed(seed, d.pre_id));
+      mt_seed(S->rng, seed);
     }
   }
   __syncthreads();
@@ -568,12 +563,10 @@ __global__ void __launch_bounds__(ACA_THREADS) aca_kernel(const DevProgram* __re
     AcaOut o;
     o.rank = rank; o.draws = draws; o.fallback = fallback; o.status = status;
     outs[d.node] = o;
-    if (rng_mode == BGP_RNG_REFERENCE) {
-      for (int q = 0; q < 624; ++q) chain_state[q] = S->rng.mt[q];
-      chain_state[624] = (uint32_t)S->rng.idx;
-      __threadfence();
-      chain_done[tk] = 1;
-    }
+    for (int q = 0; q < 624; ++q) chain_state[q] = S->rng.mt[q];
+    chain_state[624] = (uint32_t)S->rng.idx;
+    __threadfence();
+    chain_done[tk] = 1;
   }
 }
 
@@ -900,13 +893,6 @@ __global__ void dot_kernel(const double* __restrict__ a, const double* __restric
     s += a[i] * b[i];
   s = block_sum(s, red);
   if (threadIdx.x == 0) atomicAdd(out, s);
-}
-__global__ void sum_kernel(const double* __restrict__ a, int64_t n, double* out) {
-  __shared__ double red[32];
-  double s = 0.0;
-  for (int64_t i = threadIdx.x; i < n; i += blockDim.x) s += a[i];
-  s = block_sum(s, red);
-  if (threadIdx.x == 0) *out = s;
 }
 
 }  // namespace bgp

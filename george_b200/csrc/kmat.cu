@@ -375,9 +375,8 @@ static int launch_fast_nd(const FastShape& F, bool symmetric, const double* x1, 
 // returns -1 when the program has no specialised build (the caller then launches the interpreter kernels)
 static int try_launch_fast(const DevProgram& P, bool symmetric, const double* x1, int64_t n1, const double* x2, int64_t n2,
                            const double* diag_add, double* out, int64_t ld, cudaStream_t s) {
-  static const bool disabled = getenv("BGP_KMAT_GENERIC") != nullptr;  // tuning / A-B runs
   FastShape F;
-  if (disabled || !detect_fast_shape(P, &F)) return -1;
+  if (!detect_fast_shape(P, &F)) return -1;
   switch (F.shape) {
     case BGP_SHAPE_EXPSQ: return launch_fast_nd<BGP_SHAPE_EXPSQ>(F, symmetric, x1, n1, x2, n2, diag_add, out, ld, s);
     case BGP_SHAPE_M32: return launch_fast_nd<BGP_SHAPE_M32>(F, symmetric, x1, n1, x2, n2, diag_add, out, ld, s);
