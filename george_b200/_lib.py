@@ -56,17 +56,13 @@ SIGNATURES = {
     "bgp_kmat_gradient_general": (C.c_int, [_specp, _p, _p, _i64, _p, _i64, _p]),
     "bgp_kmat_x1_gradient_general": (C.c_int, [_specp, _p, _i64, _p, _i64, _p]),
     "bgp_kmat_x2_gradient_general": (C.c_int, [_specp, _p, _i64, _p, _i64, _p]),
-    "bgp_kmat_symmetric_dev": (C.c_int, [_specp, _p, _i64, _p, _p, _i64]),
-    "bgp_kmat_general_dev": (C.c_int, [_specp, _p, _i64, _p, _i64, _p, _i64]),
     "bgp_kmat_matvec": (C.c_int, [_specp, _p, _i64, _p, _i64, _p, _p, _i64, _p]),
-    "bgp_kmat_matvec_dev": (C.c_int, [_specp, _p, _i64, _p, _i64, _p, _p, _i64, _p]),
     "bgp_kmat_gradient_contract": (C.c_int, [_specp, _p, _p, _i64, _p, _p]),
     "bgp_dense_grad_terms": (C.c_int, [_p, _p, _p, _p, _p, _p]),
     "bgp_hodlr_grad_terms": (C.c_int, [_p, _p, _p, _p, _p, _p]),
     "bgp_dense_create": (C.c_int, [C.POINTER(_p)]),
     "bgp_dense_destroy": (None, [_p]),
     "bgp_dense_compute": (C.c_int, [_p, _specp, _p, _i64, _i32, _p]),
-    "bgp_dense_computed": (C.c_int, [_p]),
     "bgp_dense_log_determinant": (C.c_int, [_p, _dp]),
     "bgp_dense_apply_inverse": (C.c_int, [_p, _p, _i64, _i64]),
     "bgp_dense_dot_solve": (C.c_int, [_p, _p, _dp]),
@@ -95,23 +91,12 @@ SIGNATURES = {
     "bgp_hodlr_last_aca_profile": (C.c_int, [_p, _dp]),
     "bgp_selftest_lu": (C.c_int, [_i32, _i32, _p, _p, _p]),
     "bgp_selftest_gemm": (C.c_int, [_i32, _i32, _i32, _i32, _i32, _p, _i64, _p, _i64, _p, _i64, _i32]),
-    "bgp_hodlr_top_panel": (C.c_int, [_p, C.POINTER(_p), C.POINTER(_i64), C.POINTER(_i64), C.POINTER(_i64),
-                                      C.POINTER(_i64)]),
-    "bgp_hodlr_export_top": (C.c_int, [_p, _p, _i64]),
-    "bgp_hodlr_import_top": (C.c_int, [_p, _p, _i64]),
-    "bgp_hodlr_shard_rows": (C.c_int, [_p, _i32, C.POINTER(_i64), C.POINTER(_i64)]),
-    "bgp_hodlr_finish_top": (C.c_int, [_p]),
     "bgp_comm_unique_id": (C.c_int, [_p, C.c_char_p]),
     "bgp_comm_init": (C.c_int, [_p, C.c_int, C.c_int, C.c_char_p]),
     "bgp_comm_destroy": (C.c_int, []),
-    "bgp_comm_size": (C.c_int, []),
-    "bgp_hodlr_solve_local_dev": (C.c_int, [_p, _p, _i64, _i64]),
-    "bgp_hodlr_solve_top_dev": (C.c_int, [_p, _p, _i64, _i64]),
     "bgp_dev_alloc": (C.c_int, [C.POINTER(_p), C.c_size_t]),
     "bgp_dev_free": (C.c_int, [_p]),
     "bgp_dev_upload": (C.c_int, [_p, _p, C.c_size_t]),
-    "bgp_dev_download": (C.c_int, [_p, _p, C.c_size_t]),
-    "bgp_dev_synchronize": (C.c_int, []),
     "bgp_host_alloc_pinned": (C.c_int, [C.POINTER(_p), C.c_size_t]),
     "bgp_host_free_pinned": (C.c_int, [_p]),
 }

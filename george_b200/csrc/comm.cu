@@ -59,18 +59,9 @@ bool comm_ready() { return g_comm != nullptr && g_world > 1; }
 int comm_rank() { return g_rank; }
 int comm_world() { return g_world; }
 
-// in-place MAX all-reduce of `count` uint64 values on stream s (ncclUint64 = 5, ncclMax = 2)
-int comm_allreduce_max_u64(unsigned long long* buf, size_t count, cudaStream_t s) {
-  if (!comm_ready()) return BGP_OK;
-  const int rc = p_all_reduce(buf, buf, count, 5, 2, g_comm, s);
-  if (rc != 0) { set_error("ncclAllReduce failed: %s", p_error_string ? p_error_string(rc) : "?"); return BGP_ERR_CUDA; }
-  g_launches.fetch_add(1, std::memory_order_relaxed);
-  return BGP_OK;
-}
-
 // in-place SUM all-reduce of `count` doubles (ncclFloat64 = 8, ncclSum = 0)
 int comm_allreduce_sum_f64(double* buf, size_t count, cudaStream_t s) {
-  if (!comm_ready()) return BGP_OK;
+  if (!comm_ready()) { set_error("no communicator"); return BGP_ERR_INVALID; }
   const int rc = p_all_reduce(buf, buf, count, 8, 0, g_comm, s);
   if (rc != 0) { set_error("ncclAllReduce failed: %s", p_error_string ? p_error_string(rc) : "?"); return BGP_ERR_CUDA; }
   g_launches.fetch_add(1, std::memory_order_relaxed);
@@ -118,7 +109,5 @@ int bgp_comm_destroy(void) {
   g_comm = nullptr; g_world = 1; g_rank = 0;
   return BGP_OK;
 }
-
-int bgp_comm_size(void) { return comm_ready() ? g_world : 1; }
 
 }  // extern "C"

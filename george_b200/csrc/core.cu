@@ -285,8 +285,6 @@ int bgp_dev_alloc(void** p, size_t bytes) {
 }
 int bgp_dev_free(void* p) { BGP_CUDA(cudaFree(p)); return BGP_OK; }
 int bgp_dev_upload(void* dst, const void* src, size_t bytes) { BGP_CUDA(cudaMemcpy(dst, src, bytes, cudaMemcpyHostToDevice)); return BGP_OK; }
-int bgp_dev_download(void* dst, const void* src, size_t bytes) { BGP_CUDA(cudaMemcpy(dst, src, bytes, cudaMemcpyDeviceToHost)); return BGP_OK; }
-int bgp_dev_synchronize(void) { BGP_CUDA(cudaDeviceSynchronize()); return BGP_OK; }
 int bgp_host_alloc_pinned(void** p, size_t bytes) { BGP_CUDA(cudaMallocHost(p, bytes)); return BGP_OK; }
 int bgp_host_free_pinned(void* p) { BGP_CUDA(cudaFreeHost(p)); return BGP_OK; }
 

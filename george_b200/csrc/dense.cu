@@ -589,8 +589,6 @@ int bgp_dense_compute(bgp_dense_t* h, const bgp_kernel_spec_t* spec, const doubl
   return BGP_OK;
 }
 
-int bgp_dense_computed(const bgp_dense_t* h) { return h && h->computed ? 1 : 0; }
-
 int bgp_dense_log_determinant(const bgp_dense_t* h, double* out) {
   if (!h || !h->computed) { set_error("the solver has not been computed"); return BGP_ERR_NOT_COMPUTED; }
   *out = h->log_det;

@@ -162,9 +162,8 @@ static void build_tree(bgp_hodlr* h, int start, int size, int dir, int parent, i
   }
 }
 
-static int hodlr_solve_dev(bgp_hodlr* h, double* b, int64_t nrhs, int64_t ldb, cudaStream_t s, int part);
-static int hodlr_exchange_finish(bgp_hodlr* h);
-static int hodlr_finish_top_impl(bgp_hodlr* h, bool allreduce);
+static int hodlr_solve_dev(bgp_hodlr* h, double* b, int64_t nrhs, int64_t ldb, cudaStream_t s, bool local_only);
+static int hodlr_finish_sharded(bgp_hodlr* h);
 
 static int launch_leaf_solve(bgp_hodlr* h, double* X, int64_t ldx, const int* ncols_by_depth, int ncols_fixed,
                              int max_cols, cudaStream_t s) {
@@ -539,6 +538,11 @@ static int hodlr_compute_dev_impl(bgp_hodlr* h, const bgp_kernel_spec_t* spec, c
   if (o.shard_count & (o.shard_count - 1)) { set_error("shard_count must be a power of two"); return BGP_ERR_INVALID; }
   if (o.shard_rank < 0 || o.shard_rank >= o.shard_count) { set_error("invalid shard_rank"); return BGP_ERR_INVALID; }
   if (o.shard_count > 1 && o.rng_mode == BGP_RNG_REFERENCE) { set_error("rng_mode=reference serialises the tree and cannot be sharded"); return BGP_ERR_INVALID; }
+  if (o.shard_count > 1 && !(comm_ready() && comm_world() == o.shard_count && comm_rank() == o.shard_rank)) {
+    set_error("a sharded factorisation is collective: it needs the communicator of bgp_comm_init with world == "
+              "opts.shard_count (%d) and rank == opts.shard_rank (%d)", o.shard_count, o.shard_rank);
+    return BGP_ERR_INVALID;
+  }
   h->opts = o;
   h->n = n;
   h->ndim = ndim;
@@ -826,14 +830,9 @@ static int hodlr_compute_dev_impl(bgp_hodlr* h, const bgp_kernel_spec_t* spec, c
   }
   // (2) sharded: the factored sub-tree applied to this shard's rows of the top-level factor columns (hodlr.h:95-102 for
   //     the ancestors above the cut) — the same kernels as a solve with the top panel as right-hand sides
-  if (o.shard_count > 1 && h->top.ucols > 0) BGP_TRY(hodlr_solve_dev(h, h->top.U.p, h->top.ucols, n, sA, 1));
+  if (o.shard_count > 1 && h->top.ucols > 0) BGP_TRY(hodlr_solve_dev(h, h->top.U.p, h->top.ucols, n, sA, true));
   BGP_CUDA(cudaEventRecord(h->ev[3], sA));
-  if (o.shard_count > 1) {
-    if (comm_ready() && comm_world() == o.shard_count && comm_rank() == o.shard_rank) return hodlr_exchange_finish(h);
-    // no communicator: the caller exchanges the top panel rows itself and calls bgp_hodlr_finish_top()
-    BGP_CUDA(cudaStreamSynchronize(sA));
-    return BGP_OK;
-  }
+  if (o.shard_count > 1) return hodlr_finish_sharded(h);
 
   BGP_TRY(sum_log_det(h, sA, &h->log_det));
   h->computed = true;
@@ -879,55 +878,45 @@ static int exchange_rows(bgp_hodlr* h, double* P, int64_t ld, int64_t cols, cuda
   return BGP_OK;
 }
 
-// part: 0 = everything, 1 = local (leaves + levels >= cut), 2 = top (levels < cut)
-static int hodlr_solve_dev(bgp_hodlr* h, double* b, int64_t nrhs, int64_t ldb, cudaStream_t s, int part) {
+// local_only: the leaves and the levels at or below the shard cut, without the exchange (compute() applies the owned
+// sub-tree to the top panel this way).  Otherwise the whole solve; a sharded one all-gathers the locally solved rows
+// before the levels above the cut (replicated right-hand side: every rank needs all rows).
+static int hodlr_solve_dev(bgp_hodlr* h, double* b, int64_t nrhs, int64_t ldb, cudaStream_t s, bool local_only) {
   const int nlev = (int)h->levels.size();
-  const int cut = h->opts.shard_count > 1 ? h->cut_depth : 0;
-  const bool native_x = part == 0 && h->opts.shard_count > 1 && comm_ready() && comm_world() == h->opts.shard_count;
+  const bool sharded = h->opts.shard_count > 1;
+  const int cut = sharded ? h->cut_depth : 0;
   for (int64_t c0 = 0; c0 < nrhs; c0 += 64) {
     const int nc = (int)std::min<int64_t>(64, nrhs - c0);
     double* X = b + c0 * ldb;
-    if (part != 2) {
-      BGP_TRY(launch_leaf_solve(h, X, ldb, nullptr, nc, nc, s));
-      for (int l = nlev - 1; l >= cut; --l) BGP_TRY(launch_level(h, h->levels[l], X, ldb, nc, 0, 0, 0, nc, s));
-    }
-    if (native_x) BGP_TRY(exchange_rows(h, X, ldb, nc, s));  // replicated right-hand side: every rank needs all rows
-    if (part != 1) {
-      for (int l = std::min(cut, nlev) - 1; l >= 0; --l) BGP_TRY(launch_level(h, h->levels[l], X, ldb, nc, 0, 0, 0, nc, s));
-    }
+    BGP_TRY(launch_leaf_solve(h, X, ldb, nullptr, nc, nc, s));
+    for (int l = nlev - 1; l >= cut; --l) BGP_TRY(launch_level(h, h->levels[l], X, ldb, nc, 0, 0, 0, nc, s));
+    if (local_only) continue;
+    if (sharded) BGP_TRY(exchange_rows(h, X, ldb, nc, s));
+    for (int l = std::min(cut, nlev) - 1; l >= 0; --l) BGP_TRY(launch_level(h, h->levels[l], X, ldb, nc, 0, 0, 0, nc, s));
   }
   return BGP_OK;
 }
 
-// Gram / LU / log-det / update of the nodes above the shard cut (every rank does all of them: they are tiny), then the
-// log-determinant: owned leaves + owned nodes, the top nodes counted once (by shard 0); with `allreduce` the partial sums
-// are added over the ranks on the device (one double), otherwise log_det stays PARTIAL and the host sums over shards.
-static int hodlr_finish_top_impl(bgp_hodlr* h, bool allreduce) {
+// The collective tail of a sharded compute(): all-gather of the locally solved rows of the top-level factor panel (the
+// ONE data-path collective of compute(), SURVEY.md §8e), Gram / LU / log-det / update of the nodes above the shard cut
+// (every rank does all of them: they are tiny), then the log-determinant: owned leaves + owned nodes, the top nodes
+// counted once (by shard 0), the partial sums added over the ranks on the device (one double).
+static int hodlr_finish_sharded(bgp_hodlr* h) {
   cudaStream_t s = h->sA;
-  const int nlev = (int)h->levels.size();
-  const int cut = std::min(h->cut_depth, nlev);
+  BGP_TRY(exchange_rows(h, h->top.U.p, h->n, h->top.ucols, s));
+  const int cut = std::min(h->cut_depth, (int)h->levels.size());
   for (int l = cut - 1; l >= 0; --l) {
     const LevelInfo& L = h->levels[l];
     BGP_TRY(launch_level(h, L, h->top.U.p, h->n, L.ucol + L.r, L.ucol, 1, 0, L.ucol, s));
   }
   double ld = 0.0;
   BGP_TRY(sum_log_det(h, s, &ld));
-  if (allreduce) {
-    BGP_CUDA(cudaMemcpyAsync(h->d_scalar.p, &ld, sizeof(double), cudaMemcpyHostToDevice, s));
-    BGP_TRY(comm_allreduce_sum_f64(h->d_scalar.p, 1, s));
-    BGP_CUDA(cudaMemcpyAsync(&ld, h->d_scalar.p, sizeof(double), cudaMemcpyDeviceToHost, s));
-    BGP_CUDA(cudaStreamSynchronize(s));
-  }
+  BGP_CUDA(cudaMemcpyAsync(h->d_scalar.p, &ld, sizeof(double), cudaMemcpyHostToDevice, s));
+  BGP_TRY(comm_allreduce_sum_f64(h->d_scalar.p, 1, s));
+  BGP_CUDA(cudaMemcpyAsync(&ld, h->d_scalar.p, sizeof(double), cudaMemcpyDeviceToHost, s));
+  BGP_CUDA(cudaStreamSynchronize(s));
   h->log_det = ld;
   h->computed = true;
-  return BGP_OK;
-}
-
-// sharded compute with the library's communicator: all-gather of the locally solved rows of the top-level factor panel
-// (the ONE data-path collective of compute(), SURVEY.md §8e), then the top nodes, then the log-det all-reduce.
-static int hodlr_exchange_finish(bgp_hodlr* h) {
-  BGP_TRY(exchange_rows(h, h->top.U.p, h->n, h->top.ucols, h->sA));
-  BGP_TRY(hodlr_finish_top_impl(h, true));
   record_compute_timing(h);
   return BGP_OK;
 }
@@ -993,7 +982,7 @@ int bgp_hodlr_apply_inverse(bgp_hodlr_t* h, double* b, int64_t nrhs, int64_t ldb
     const int64_t nc = std::min(slab, nrhs - c0);
     BGP_CUDA(cudaMemcpy2DAsync(h->d_rhs.p, sizeof(double) * n, b + c0 * ldb, sizeof(double) * ldb, sizeof(double) * n, nc, cudaMemcpyHostToDevice, s));
     BGP_CUDA(cudaEventRecord(h->ev[4], s));
-    BGP_TRY(hodlr_solve_dev(h, h->d_rhs.p, nc, n, s, 0));
+    BGP_TRY(hodlr_solve_dev(h, h->d_rhs.p, nc, n, s, false));
     BGP_CUDA(cudaEventRecord(h->ev[5], s));
     BGP_CUDA(cudaMemcpy2DAsync(b + c0 * ldb, sizeof(double) * ldb, h->d_rhs.p, sizeof(double) * n, sizeof(double) * n, nc, cudaMemcpyDeviceToHost, s));
     BGP_CUDA(cudaStreamSynchronize(s));
@@ -1009,7 +998,7 @@ int bgp_hodlr_dot_solve_dev(bgp_hodlr_t* h, const double* y_dev, double* out) {
   BGP_TRY(h->d_rhs.reserve((size_t)n, s));
   BGP_CUDA(cudaEventRecord(h->ev[4], s));
   BGP_CUDA(cudaMemcpyAsync(h->d_rhs.p, y_dev, sizeof(double) * n, cudaMemcpyDeviceToDevice, s));
-  BGP_TRY(hodlr_solve_dev(h, h->d_rhs.p, 1, n, s, 0));
+  BGP_TRY(hodlr_solve_dev(h, h->d_rhs.p, 1, n, s, false));
   BGP_CUDA(cudaMemsetAsync(h->d_scalar.p, 0, sizeof(double), s));
   dot_kernel<<<(unsigned)std::min<int64_t>((n + 255) / 256, 592), 256, 0, s>>>(y_dev, h->d_rhs.p, n, h->d_scalar.p);
   BGP_LAUNCH_CHECK();
@@ -1055,11 +1044,11 @@ int bgp_hodlr_grad_terms(bgp_hodlr_t* h, const uint32_t* which, const double* r,
   double* dg = h->d_rhs.p + n;
   double* ddiag = h->d_rhs.p + n + 64;
   BGP_CUDA(cudaMemcpyAsync(alpha, r, sizeof(double) * n, cudaMemcpyHostToDevice, s));
-  BGP_TRY(hodlr_solve_dev(h, alpha, 1, n, s, 0));
+  BGP_TRY(hodlr_solve_dev(h, alpha, 1, n, s, false));
   if (alpha_out) BGP_CUDA(cudaMemcpyAsync(alpha_out, alpha, sizeof(double) * n, cudaMemcpyDeviceToHost, s));
   BGP_TRY(h->d_inv.reserve((size_t)n * n, s));
   BGP_TRY(fill_identity_launch(h->d_inv.p, n, s));
-  BGP_TRY(hodlr_solve_dev(h, h->d_inv.p, n, n, s, 0));
+  BGP_TRY(hodlr_solve_dev(h, h->d_inv.p, n, n, s, false));
   BGP_TRY(h->d_which.reserve(std::max(np, 1), s));
   if (np) BGP_CUDA(cudaMemcpyAsync(h->d_which.p, which, sizeof(unsigned) * np, cudaMemcpyHostToDevice, s));
   BGP_TRY(kmat_grad_contract_launch(h->d_prog.p, h->ndim, np, h->d_which.p, h->d_x.p, n, h->d_inv.p, n, alpha, 1.0, -1.0, dg,
@@ -1164,66 +1153,6 @@ int bgp_selftest_gemm(int32_t a_kcontig, int32_t b_kcontig, int32_t m, int32_t n
   else { set_error("bgp_selftest_gemm: only the (A K-contiguous | M-contiguous) x (B K-contiguous) variants are built here"); return BGP_ERR_INVALID; }
   BGP_CUDA(cudaMemcpyAsync(C_host, dC.p, sizeof(double) * nc, cudaMemcpyDeviceToHost, s));
   BGP_CUDA(cudaStreamSynchronize(s));
-  return BGP_OK;
-}
-
-// ---- multi-GPU exchange (SURVEY.md §8e) -----------------------------------------------------------------------
-int bgp_hodlr_top_panel(bgp_hodlr_t* h, double** ptr_dev, int64_t* row0, int64_t* rows, int64_t* cols, int64_t* ld) {
-  if (!h) { set_error("null handle"); return BGP_ERR_INVALID; }
-  *ptr_dev = h->top.U.p;
-  *row0 = h->row0; *rows = h->nloc;
-  *cols = h->top.ucols;
-  *ld = h->n;
-  return BGP_OK;
-}
-
-
-int bgp_hodlr_shard_rows(const bgp_hodlr_t* h, int32_t s, int64_t* row0, int64_t* rows) {
-  if (!h || s < 0 || s >= (int)h->shard_rows.size()) { set_error("shard index out of range"); return BGP_ERR_INDEX; }
-  *row0 = h->shard_row0[s]; *rows = h->shard_rows[s];
-  return BGP_OK;
-}
-
-int bgp_hodlr_export_top(bgp_hodlr_t* h, double* buf_dev, int64_t rows_pad) {
-  if (!h) { set_error("null handle"); return BGP_ERR_INVALID; }
-  const int64_t cols = h->top.ucols;
-  if (cols == 0 || h->nloc == 0) return BGP_OK;
-  if (rows_pad < h->nloc) { set_error("rows_pad too small"); return BGP_ERR_INVALID; }
-  pack_rows_kernel<<<1184, 256, 0, h->sA>>>(h->top.U.p, h->n, h->row0, h->nloc, cols, buf_dev, rows_pad);
-  BGP_LAUNCH_CHECK();
-  BGP_CUDA(cudaStreamSynchronize(h->sA));
-  return BGP_OK;
-}
-
-int bgp_hodlr_import_top(bgp_hodlr_t* h, const double* all_buf_dev, int64_t rows_pad) {
-  if (!h) { set_error("null handle"); return BGP_ERR_INVALID; }
-  const int64_t cols = h->top.ucols;
-  if (cols == 0) return BGP_OK;
-  for (size_t s = 0; s < h->shard_rows.size(); ++s) {
-    if ((int)s == h->opts.shard_rank) continue;  // own rows are already in place
-    unpack_rows_kernel<<<1184, 256, 0, h->sA>>>(h->top.U.p, h->n, h->shard_row0[s], h->shard_rows[s], cols,
-                                                all_buf_dev + (int64_t)s * cols * rows_pad, rows_pad);
-    BGP_LAUNCH_CHECK();
-  }
-  BGP_CUDA(cudaStreamSynchronize(h->sA));
-  return BGP_OK;
-}
-
-int bgp_hodlr_finish_top(bgp_hodlr_t* h) {
-  if (!h) { set_error("null handle"); return BGP_ERR_INVALID; }
-  return hodlr_finish_top_impl(h, false);
-}
-
-int bgp_hodlr_solve_local_dev(bgp_hodlr_t* h, double* b_dev, int64_t nrhs, int64_t ldb) {
-  if (!h || !h->computed) { set_error("the solver has not been computed"); return BGP_ERR_NOT_COMPUTED; }
-  BGP_TRY(hodlr_solve_dev(h, b_dev, nrhs, ldb, h->sA, 1));
-  BGP_CUDA(cudaStreamSynchronize(h->sA));
-  return BGP_OK;
-}
-int bgp_hodlr_solve_top_dev(bgp_hodlr_t* h, double* b_dev, int64_t nrhs, int64_t ldb) {
-  if (!h || !h->computed) { set_error("the solver has not been computed"); return BGP_ERR_NOT_COMPUTED; }
-  BGP_TRY(hodlr_solve_dev(h, b_dev, nrhs, ldb, h->sA, 2));
-  BGP_CUDA(cudaStreamSynchronize(h->sA));
   return BGP_OK;
 }
 

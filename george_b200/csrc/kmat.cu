@@ -573,23 +573,4 @@ int bgp_kmat_gradient_general(const bgp_kernel_spec_t* spec, const uint32_t* whi
   return kmat_grad_host(spec, which, x1, n1, x2, n2, out, 0);
 }
 
-int bgp_kmat_symmetric_dev(const bgp_kernel_spec_t* spec, const double* x_dev, int64_t n, const double* diag_add_dev,
-                           double* out_dev, int64_t ld) {
-  BGP_TRY(require_device());
-  DevProgram P;
-  BGP_TRY(build_dev_program(spec, &P));
-  DevBuf<DevProgram> dprog;
-  BGP_TRY(upload_program(P, dprog, 0));
-  return kmat_symmetric_launch_auto(P, dprog.p, x_dev, n, diag_add_dev, out_dev, ld, 0);
-}
-int bgp_kmat_general_dev(const bgp_kernel_spec_t* spec, const double* x1_dev, int64_t n1, const double* x2_dev,
-                         int64_t n2, double* out_dev, int64_t ld) {
-  BGP_TRY(require_device());
-  DevProgram P;
-  BGP_TRY(build_dev_program(spec, &P));
-  DevBuf<DevProgram> dprog;
-  BGP_TRY(upload_program(P, dprog, 0));
-  return kmat_general_launch_auto(P, dprog.p, x1_dev, n1, x2_dev, n2, out_dev, ld, 0);
-}
-
 }  // extern "C"

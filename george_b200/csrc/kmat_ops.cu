@@ -315,21 +315,6 @@ int bgp_kmat_matvec(const bgp_kernel_spec_t* spec, const double* x1, int64_t n1,
   return BGP_OK;
 }
 
-int bgp_kmat_matvec_dev(const bgp_kernel_spec_t* spec, const double* x1_dev, int64_t n1, const double* x2_dev, int64_t n2,
-                        const double* diag_dev, const double* v_dev, int64_t nrhs, double* out_dev) {
-  BGP_TRY(require_device());
-  DevProgram P;
-  BGP_TRY(build_dev_program(spec, &P));
-  if (n1 < 0 || n2 < 0 || nrhs < 0) { set_error("negative size"); return BGP_ERR_INVALID; }
-  if (diag_dev && n1 != n2) { set_error("dimension mismatch: a diagonal term needs a square operator"); return BGP_ERR_DIM; }
-  DevBuf<DevProgram> dprog;
-  DevBuf<double> scratch;
-  BGP_TRY(upload_program(P, dprog, 0));
-  BGP_TRY(kmat_matvec_launch(dprog.p, P.ndim, x1_dev, n1, x2_dev, n2, diag_dev, v_dev, n2, nrhs, out_dev, n1, scratch, 0));
-  BGP_CUDA(cudaStreamSynchronize(0));
-  return BGP_OK;
-}
-
 int bgp_kmat_gradient_contract(const bgp_kernel_spec_t* spec, const uint32_t* which, const double* x, int64_t n,
                                const double* A, double* out) {
   BGP_TRY(require_device());

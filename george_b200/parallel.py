@@ -17,8 +17,6 @@ The reference has no distributed code; what shards is the algorithmic independen
 vector, top nodes redundantly.  ``torch.distributed`` is plumbing only: it broadcasts the 128-byte NCCL unique id with
 which every rank initialises the library's communicator (``ensure_device_comm``).  All arithmetic and all data-path
 collectives are in ``csrc/hodlr.cu`` / ``csrc/comm.cu``.
-
-The exchange helpers at the bottom are backend-agnostic (tested with gloo on CPU tensors in ``tests/test_parallel.py``).
 """
 
 import ctypes as C
@@ -28,7 +26,7 @@ import numpy as np
 from . import _lib
 from ._spec import flatten
 
-__all__ = ["ShardedHODLRSolver", "shard_ranges", "allgather_padded"]
+__all__ = ["ShardedHODLRSolver", "shard_ranges"]
 
 
 def shard_ranges(n, shard_count, min_size):
@@ -49,23 +47,6 @@ def shard_ranges(n, shard_count, min_size):
             nxt.append((start + half, size - half))
         level = nxt
     return level
-
-
-def allgather_padded(local, rows_pad, group=None):
-    """All-gather 2-D blocks ``local`` (cols x rows_i, last dim contiguous) whose row counts differ by at most a few:
-    every rank pads to ``rows_pad`` and the result has shape ``(world, cols, rows_pad)``."""
-    import torch
-    import torch.distributed as dist
-    world = dist.get_world_size(group)
-    cols, rows = local.shape
-    send = local
-    if rows != rows_pad:
-        send = torch.zeros((cols, rows_pad), dtype=local.dtype, device=local.device)
-        send[:, :rows] = local
-    send = send.contiguous()
-    out = torch.empty((world, cols, rows_pad), dtype=local.dtype, device=local.device)
-    dist.all_gather_into_tensor(out.view(-1), send.view(-1), group=group)
-    return out
 
 
 _COMM_WORLD = 0

@@ -115,8 +115,6 @@ int bgp_spec_num_params(const bgp_kernel_spec_t* spec, int* n_params);
  * (src/george/kernel_interface.cpp:62-77, 47-60, 79-90) and gradient_symmetric / gradient_general
  * (kernel_interface.cpp:109-125, 92-107).  x1: (n1, ndim) row-major f64; out row-major f64.
  * `which` (n_params uint32) selects the hyper-parameters to differentiate; unselected slices are 0.
- * The *_dev variants take device pointers and run on the handle-less default stream of the
- * calling thread's device; they are what the solvers call internally.
  * ------------------------------------------------------------------------------------------ */
 int bgp_kmat_symmetric(const bgp_kernel_spec_t* spec, const double* x, int64_t n, double* out /* n*n */);
 int bgp_kmat_general(const bgp_kernel_spec_t* spec, const double* x1, int64_t n1, const double* x2, int64_t n2,
@@ -133,12 +131,6 @@ int bgp_kmat_x1_gradient_general(const bgp_kernel_spec_t* spec, const double* x1
                                  int64_t n2, double* out /* n1*n2*ndim */);
 int bgp_kmat_x2_gradient_general(const bgp_kernel_spec_t* spec, const double* x1, int64_t n1, const double* x2,
                                  int64_t n2, double* out /* n1*n2*ndim */);
-/* device-resident build: out_dev[i*ld + j] (row-major, ld >= n2); diag_add_dev (may be NULL, symmetric only)
- * is added on the diagonal — the fusion of solvers/basic.py:64-65. */
-int bgp_kmat_symmetric_dev(const bgp_kernel_spec_t* spec, const double* x_dev, int64_t n, const double* diag_add_dev,
-                           double* out_dev, int64_t ld);
-int bgp_kmat_general_dev(const bgp_kernel_spec_t* spec, const double* x1_dev, int64_t n1, const double* x2_dev,
-                         int64_t n2, double* out_dev, int64_t ld);
 
 /* ------------------------------------------------------------------------------------------
  * Matrix-free consumers of the covariance function (csrc/kmat_ops.cu): the kernel matrix is never formed.
@@ -154,8 +146,6 @@ int bgp_kmat_general_dev(const bgp_kernel_spec_t* spec, const double* x1_dev, in
  * ------------------------------------------------------------------------------------------ */
 int bgp_kmat_matvec(const bgp_kernel_spec_t* spec, const double* x1, int64_t n1, const double* x2, int64_t n2,
                     const double* diag, const double* v, int64_t nrhs, double* out);
-int bgp_kmat_matvec_dev(const bgp_kernel_spec_t* spec, const double* x1_dev, int64_t n1, const double* x2_dev,
-                        int64_t n2, const double* diag_dev, const double* v_dev, int64_t nrhs, double* out_dev);
 int bgp_kmat_gradient_contract(const bgp_kernel_spec_t* spec, const uint32_t* which, const double* x, int64_t n,
                                const double* A, double* out /* n_params */);
 
@@ -169,7 +159,6 @@ void bgp_dense_destroy(bgp_dense_t* h);
 /* basic.py:51-70.  yerr is the standard deviation; yerr^2 is added on the diagonal. */
 int bgp_dense_compute(bgp_dense_t* h, const bgp_kernel_spec_t* spec, const double* x, int64_t n, int32_t ndim,
                       const double* yerr);
-int bgp_dense_computed(const bgp_dense_t* h);
 int bgp_dense_log_determinant(const bgp_dense_t* h, double* out);
 /* basic.py:72-87.  b: (n, nrhs) column-major with leading dimension ldb (a plain vector has nrhs=1); in place. */
 int bgp_dense_apply_inverse(bgp_dense_t* h, double* b, int64_t nrhs, int64_t ldb);
@@ -280,8 +269,7 @@ int bgp_hodlr_last_work(const bgp_hodlr_t* h, double* w6);
  * [2] candidate-row entries verified against the 1e-14 pivot threshold (hodlr.h:191), [3] residual-update FMAs,
  * [4] candidate rows examined, [5] entries of [2] that were actually evaluated (the others were bounded below the
  * threshold from the kernel's decay and the factor magnitudes, without evaluation; decisions are identical),
- * [6..11] summed launch times ms of a2_eval (+ its all-reduce when sharded), a2_decide, a2_vrow, a2_pivot,
- * a2_vnorm_ucol, a2_finish. */
+ * [6..11] summed launch times ms of a2_eval, a2_decide, a2_vrow, a2_pivot, a2_vnorm_ucol, a2_finish. */
 int bgp_hodlr_set_profiling(bgp_hodlr_t* h, int on);
 int bgp_hodlr_last_aca_profile(const bgp_hodlr_t* h, double* p12);
 
@@ -296,32 +284,18 @@ int bgp_selftest_lu(int32_t n, int32_t nrhs, const double* S_host, double* R_hos
 int bgp_selftest_gemm(int32_t a_kcontig, int32_t b_kcontig, int32_t m, int32_t n, int32_t k, const double* A_host,
                       int64_t lda, const double* B_host, int64_t ldb, double* C_host, int64_t ldc, int32_t atomic_add);
 
-/* Multi-GPU (SURVEY.md §8e).  With a communicator (bgp_comm_init) whose size and rank match opts.shard_count /
- * opts.shard_rank, bgp_hodlr_compute[_dev] is COLLECTIVE and complete: local sub-tree, all-gather of the rows this shard
- * owns of the top-level factor panel (pack kernel -> ncclAllGather -> unpack kernels on the solver's stream), the nodes
- * above the cut, log-det all-reduce; apply_inverse / dot_solve are collective too (replicated right-hand side, one
- * all-gather of the locally solved slices).  WITHOUT a communicator the same steps are exposed one by one so that a host
- * can run the exchange itself: the rows are exported, all-gathered by the host, imported, and the top nodes finished.
- *   bgp_hodlr_top_panel(h, &ptr_dev, &rows, &cols, &ld): device pointer to the (N x cols) column-major panel
- *   bgp_hodlr_finish_top(h): Gram/LU/log-det/update of the nodes above the shard cut.               */
-int bgp_hodlr_top_panel(bgp_hodlr_t* h, double** ptr_dev, int64_t* row0, int64_t* rows, int64_t* cols, int64_t* ld);
-/* pack this shard's rows of the top panel into a contiguous (cols x rows_pad) device buffer (column c at c*rows_pad),
- * and scatter the all-gathered buffers (shard s at s*cols*rows_pad) of all shards back into the panel. */
-int bgp_hodlr_export_top(bgp_hodlr_t* h, double* buf_dev, int64_t rows_pad);
-int bgp_hodlr_import_top(bgp_hodlr_t* h, const double* all_buf_dev, int64_t rows_pad);
-/* row range [row0, row0+rows) owned by shard `s` (same on every shard; -1 rows if the tree cannot be cut) */
-int bgp_hodlr_shard_rows(const bgp_hodlr_t* h, int32_t s, int64_t* row0, int64_t* rows);
-int bgp_hodlr_finish_top(bgp_hodlr_t* h);
-/* The library's NCCL communicator (one per process).  Rank 0 makes a unique id (128 bytes), the host broadcasts it over
- * whatever it has (torch.distributed, MPI, a file), every rank calls bgp_comm_init.  `nccl_path` may be NULL: the library
- * already loaded in the process (torch's libnccl.so.2) is used, else libnccl.so.2 is dlopen'ed. */
+/* Multi-GPU (SURVEY.md §8e).  A factorisation with opts.shard_count > 1 is COLLECTIVE: it needs the library's
+ * communicator (bgp_comm_init) with world == opts.shard_count and rank == opts.shard_rank, and bgp_hodlr_compute[_dev]
+ * fails with BGP_ERR_INVALID without one.  Each rank factors its local sub-tree, the ranks all-gather the rows each owns
+ * of the top-level factor panel (pack kernel -> ncclAllGather -> unpack kernels on the solver's stream), every rank
+ * finishes the nodes above the cut, and the log-det is all-reduced.  apply_inverse / dot_solve on such a handle are
+ * collective too (replicated right-hand side, one all-gather of the locally solved slices).
+ * The communicator is one per process.  Rank 0 makes a unique id (128 bytes), the host broadcasts it over whatever it
+ * has (torch.distributed, MPI, a file), every rank calls bgp_comm_init.  `nccl_path` may be NULL: the library already
+ * loaded in the process (torch's libnccl.so.2) is used, else libnccl.so.2 is dlopen'ed. */
 int bgp_comm_unique_id(void* out128, const char* nccl_path);
 int bgp_comm_init(const void* id128, int rank, int world, const char* nccl_path);
 int bgp_comm_destroy(void);
-int bgp_comm_size(void);
-/* sharded solve: local part, then (host all-gathers the vector), then top part. */
-int bgp_hodlr_solve_local_dev(bgp_hodlr_t* h, double* b_dev, int64_t nrhs, int64_t ldb);
-int bgp_hodlr_solve_top_dev(bgp_hodlr_t* h, double* b_dev, int64_t nrhs, int64_t ldb);
 
 /* ------------------------------------------------------------------------------------------
  * Device memory helpers so a host without torch can stage inputs (bench "value" leg).
@@ -329,8 +303,6 @@ int bgp_hodlr_solve_top_dev(bgp_hodlr_t* h, double* b_dev, int64_t nrhs, int64_t
 int bgp_dev_alloc(void** ptr_dev, size_t bytes);
 int bgp_dev_free(void* ptr_dev);
 int bgp_dev_upload(void* dst_dev, const void* src_host, size_t bytes);
-int bgp_dev_download(void* dst_host, const void* src_dev, size_t bytes);
-int bgp_dev_synchronize(void);
 int bgp_host_alloc_pinned(void** ptr, size_t bytes);
 int bgp_host_free_pinned(void* ptr);
 

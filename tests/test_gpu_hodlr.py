@@ -160,6 +160,17 @@ def test_strange_hodlr_bug(gpu):
     gp_hodlr.log_likelihood(y[:n])
 
 
+def test_sharded_compute_without_communicator_is_refused(gpu):
+    """A sharded factorisation is collective: without the library's communicator it must fail up front, not return a
+    handle that is uncomputed or holds one shard's partial log-determinant."""
+    from george_b200.solvers._hodlr import HODLRSolver
+    kernel, x, yerr = _setup_solver_test()
+    s = HODLRSolver()
+    with pytest.raises(ValueError, match="communicator"):
+        s.compute(kernel, x, yerr, min_size=100, tol=1e-10, shard_rank=0, shard_count=2)
+    assert s.computed == 0
+
+
 def test_docs_golden_loglikelihood(gpu):
     """docs/tutorials/scaling.rst:56-91: log-likelihood 133.946394912 for both solvers at N=100."""
     import george_b200 as george
